@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: impressions/sec scored (BASELINE.json `metric`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of scripts/eval.py's FinalAttentionComponent.transform over the rank's shard
@@ -64,7 +64,9 @@ WORKLOAD = ("MIND-large-shaped eval (BASELINE configs[3]): FinalAttention user e
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline (and of --workload cfg5); the secondary legs reported under "
+                         "their own keys keep their own step counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["native", "reference", "reference-gpu"], default="native")
     ap.add_argument("--impressions", type=int, default=2_400_000, help="impressions per rank per step")
@@ -85,7 +87,18 @@ def parse_args():
                          "else dma; none = transform only, for diagnosis: results invalid)")
     ap.add_argument("--chunk-rows", type=int, default=0, help="cfg5: table rows transformed + pushed per chunk")
     ap.add_argument("--strong-chunks", type=int, default=4, help="strong leg: chunks per rank of the row transform")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's scores and dense ranks of the last timed step (a fixed, "
+                         "seeded sample of whole impressions, at most 64 MB) as DIR/<name>.npy, so that two builds "
+                         "can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native path (--impl native)")
+    if args.dump_outputs and args.only_stage_a:
+        ap.error("--dump-outputs writes the headline step's outputs, which --only-stage-a does not run")
+    return args
 
 
 def measured_peaks():
@@ -180,6 +193,31 @@ def make_device_labels(c_off: torch.Tensor, seed: int, device) -> torch.Tensor:
         nxt = c_off[:-1][full] + (pos[full] - c_off[:-1][full] + 1) % cnt[full]
         lab[nxt] = 0
     return lab
+
+
+DUMP_MAX_CANDIDATES = 4_000_000  # scores + ranks in float32: 32 MB
+
+
+def dump_outputs(out_dir: str, scores: torch.Tensor, ranks: torch.Tensor, c_off: torch.Tensor):
+    """Write what a step returned to its caller -- per-candidate scores and dense ranks -- for whole impressions
+    drawn in a seeded random order until DUMP_MAX_CANDIDATES candidates are taken, stored in ascending impression
+    order.  The inputs are seeded, so two builds run with the same arguments dump the same positions."""
+    n_imp = c_off.numel() - 1
+    counts = (c_off[1:] - c_off[:-1]).cpu()
+    order = torch.randperm(n_imp, generator=torch.Generator().manual_seed(0))
+    keep = int(torch.searchsorted(torch.cumsum(counts[order], 0), DUMP_MAX_CANDIDATES, right=True))
+    imp = order[:max(keep, 1)].sort().values
+    cnt = counts[imp]
+    first = c_off[:-1].cpu()[imp]
+    local = torch.arange(int(cnt.sum())) - torch.repeat_interleave(torch.cumsum(cnt, 0) - cnt, cnt)
+    pos = (torch.repeat_interleave(first, cnt) + local).to(scores.device)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"scores": scores[pos].float(), "ranks": ranks[pos].float(),
+              "impressions": imp.double(), "candidates_per_impression": cnt.double()}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+    print("bench: wrote %s/{%s}.npy (%d impressions, %d candidates)" % (out_dir, ",".join(arrays), imp.numel(),
+                                                                      pos.numel()), file=sys.stderr, flush=True)
 
 
 def _ev():
@@ -313,6 +351,8 @@ def run_native(args):
     launches = lib.nrb_kernel_launches() - launches0
     clocks = sampler.stop() if rank == 0 else None
     ops.raise_on_index_error(flag, "bench")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, scores, ranks, c_off)
     kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in kev]))
     ms_step = D.max_ms(ms_total) / args.steps
     value = n_imp * world / (ms_step * 1e-3)
@@ -634,6 +674,8 @@ def leg_cfg5(args, D, peaks, standalone: bool = False):
     clocks = sampler.stop() if rank == 0 else None
     launches = lib.nrb_kernel_launches() - launches0
     ops.raise_on_index_error(flag, "bench cfg5")
+    if standalone and args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, scores, ranks, c_off)
     ms_step = D.max_ms(t0.elapsed_time(t1)) / steps
     build_ms = float(np.mean([a.elapsed_time(b) for a, b, _ in kev]))
     score_ms = float(np.mean([b.elapsed_time(c) for _, b, c in kev]))

@@ -54,6 +54,29 @@ def golden_latent(ref, name, dim, L, B, S, seed):
     print(name, pooled.shape, float(pooled.norm(dim=-1).mean()))
 
 
+def golden_latent_short_masks(ref):
+    """d=256, 32 latents, token masks as short as one token (min_len=1: lengths 6, 6, 4), pooled by the reference;
+    plus the digests of d=256 checkpoints (FinalAttention hidden 4096, LatentAttentionModel 64 latents) that the
+    reference's modules load strictly, for the checkpoint-factory test."""
+    dim, L, seed = 256, 32, 11
+    model = ref_harness.make_reference_latent_model(ref, dim, L, seed=seed)
+    sd = syn.make_latent_state_dict(dim, L, seed=seed)
+    model.load_state_dict(sd, strict=True)
+    x, mask = syn.make_token_batch(3, 9, dim, seed=12, min_len=1)
+    with torch.no_grad():
+        pooled = model(x, mask)
+    fa_sd = syn.make_final_attention_state_dict(dim, 4096, seed=dim)
+    ref_harness.make_reference_final_attention(ref, dim, 4096, seed=dim).load_state_dict(fa_sd, strict=True)
+    lat_sd = syn.make_latent_state_dict(dim, 64, seed=dim + 1)
+    ref_harness.make_reference_latent_model(ref, dim, 64, seed=dim + 1).load_state_dict(lat_sd, strict=True)
+    np.savez_compressed(
+        os.path.join(GOLD, "latent_short_masks_d256_L32.npz"),
+        dim=dim, L=L, seed=seed, sd_sha256=sd_digest(sd), mask_len=mask.sum(1).numpy(), pooled=pooled.numpy(),
+        final_attention_h4096_sha256=sd_digest(fa_sd), latent_L64_sha256=sd_digest(lat_sd),
+    )
+    print("latent_short_masks_d256_L32", pooled.shape, mask.sum(1).tolist())
+
+
 def golden_final(ref, name, dim, hidden, n_rows, n_imp, cand, seed, users_kept=None):
     model = ref_harness.make_reference_final_attention(ref, dim, hidden, seed=seed)
     sd = syn.make_final_attention_state_dict(dim, hidden, seed=seed)
@@ -201,6 +224,8 @@ def main():
             golden_final(ref, "final_medium_d1024", 1024, 4096, 20000, 1024, "large", seed=7, users_kept=32)
         if "latent_user_cfg5_d1024_L1024_H200" in only:
             golden_latent_user_encoder(ref, "latent_user_cfg5_d1024_L1024_H200", 1024, 1024, 3000, 20, 200, seed=777)
+        if "latent_short_masks_d256_L32" in only:
+            golden_latent_short_masks(ref)
         return
     golden_small(ref)
     golden_new_attention(ref)
@@ -214,6 +239,7 @@ def main():
     # BASELINE configs[4] shapes (d=1024, 1024 latents, histories up to 200)
     golden_latent(ref, "latent_cfg5_d1024_L1024", 1024, 1024, 4, 24, seed=555)
     golden_latent_user_encoder(ref, "latent_user_cfg5_d1024_L1024_H200", 1024, 1024, 3000, 20, 200, seed=777)
+    golden_latent_short_masks(ref)
 
 
 if __name__ == "__main__":

@@ -99,34 +99,35 @@ def test_state_dict_keys_match_reference(golden_dir):
         [f"linear{i}.weight" for i in range(1, 6)] + [f"linear{i}.bias" for i in range(1, 5)])
 
 
-def test_reference_checkpoints_load_through_the_factories(tmp_path, monkeypatch):
-    """torch.save(reference_module.state_dict()) -> get_*_model(path) (modeling_utils.py:151-155, 274-279): strict
-    load, every tensor identical, eval mode.  Needs the reference tree (this container); loading needs no GPU."""
-    from oracle import ref_harness
-    if not ref_harness.reference_available():
-        pytest.skip("/root/reference not present (GPU box)")
-    from news_recommendation_project_v2_b200 import config, modeling_utils as mu
-    ref = ref_harness.load_reference()
+def test_reference_checkpoints_load_through_the_factories(golden_dir, tmp_path, monkeypatch):
+    """torch.save(state_dict in the reference's layout) -> get_*_model(path) (modeling_utils.py:151-155, 274-279):
+    strict load, every tensor identical, eval mode.  The checkpoints are the synthetic weights that the reference's own
+    modules loaded strictly when the golden vectors were minted (oracle/make_golden.py), pinned by the weight digests
+    stored with those vectors."""
+    from news_recommendation_project_v2_b200 import config, modeling_utils as mu, synthetic as syn
+    from oracle.make_golden import sd_digest
     monkeypatch.setattr(config, "DEVICE", torch.device("cpu"))
-    for dim in (256, 1024):
+    for name, factory in (("final_small_d768", mu.get_final_attention_model),
+                          ("final_large_d1024", mu.get_final_attention_model),
+                          ("latent_default_d1024_L64", mu.get_latent_attention_model)):
+        g = np.load(os.path.join(golden_dir, name + ".npz"))
+        dim, seed = int(g["dim"]), int(g["seed"])
         monkeypatch.setattr(config, "REDUCED_DIM", dim)
         monkeypatch.setattr(config, "EMBEDDING_DIM", dim)
-        ref_fa = ref_harness.make_reference_final_attention(ref, dim, 4096, seed=dim)
-        p = tmp_path / f"fa_{dim}.pt"
-        torch.save(ref_fa.state_dict(), p)
-        ours = mu.get_final_attention_model(p)
-        assert not ours.training
-        for k, v in ref_fa.state_dict().items():
-            assert torch.equal(ours.state_dict()[k], v), k
-        ref_lat = ref_harness.make_reference_latent_model(ref, dim, 64, seed=dim + 1)
-        p = tmp_path / f"lat_{dim}.pt"
-        torch.save(ref_lat.state_dict(), p)
-        ours = mu.get_latent_attention_model(p)
-        assert not ours.training and set(ours.state_dict()) == set(ref_lat.state_dict())
-        for k, v in ref_lat.state_dict().items():
+        if factory is mu.get_final_attention_model:
+            sd = syn.make_final_attention_state_dict(dim, int(g["hidden"]), seed=seed)
+        else:
+            sd = syn.make_latent_state_dict(dim, int(g["L"]), seed=seed)
+            assert sorted(sd) == list(g["keys"])
+        assert sd_digest(sd) == str(g["sd_sha256"]), name
+        p = tmp_path / f"{name}.pt"
+        torch.save(sd, p)
+        ours = factory(p)
+        assert not ours.training and set(ours.state_dict()) == set(sd)
+        for k, v in sd.items():
             assert torch.equal(ours.state_dict()[k], v), k
     with pytest.raises(RuntimeError):
-        mu.get_latent_attention_model(tmp_path / "fa_1024.pt")  # wrong architecture: strict load refuses
+        mu.get_latent_attention_model(tmp_path / "final_large_d1024.pt")  # wrong architecture: strict load refuses
 
 
 def test_group_items_pad_and_rank_object_arrays():
@@ -346,6 +347,44 @@ def test_bench_reference_arm_contract():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=root, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+    # argument errors are refused before any work
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"], ["--only-stage-a", "--dump-outputs", "x"]):
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), *bad], capture_output=True, text=True,
+                             timeout=600, cwd=root)
+        assert out.returncode == 2 and out.stdout == "", out.stderr[-2000:]
+
+
+def test_bench_dump_outputs_sample(tmp_path):
+    """`bench.py --dump-outputs`: whole impressions of a seeded sample, in ascending order, scores and ranks at their
+    candidates' positions, float32 / float64 files, within the candidate budget, the same sample on every call."""
+    import bench
+    g = torch.Generator().manual_seed(1)
+    for n_imp in (7, 300_000):
+        cnt = torch.randint(2, 301, (n_imp,), generator=g)
+        c_off = torch.cat([torch.zeros(1, dtype=torch.int64), torch.cumsum(cnt, 0)])
+        n_c = int(c_off[-1])
+        scores = torch.randn(n_c, generator=g)
+        ranks = torch.randint(1, 301, (n_c,), generator=g, dtype=torch.int32)
+        dumps = []
+        for run in range(2):
+            d = tmp_path / f"{n_imp}_{run}"
+            bench.dump_outputs(str(d), scores, ranks, c_off)
+            dumps.append({f.stem: np.load(f) for f in d.glob("*.npy")})
+        a = dumps[0]
+        assert set(a) == {"scores", "ranks", "impressions", "candidates_per_impression"}
+        for k in a:
+            assert a[k].dtype in (np.float32, np.float64) and np.array_equal(a[k], dumps[1][k])
+        imp = a["impressions"].astype(np.int64)
+        assert np.all(np.diff(imp) > 0) and np.array_equal(a["candidates_per_impression"], cnt.numpy()[imp])
+        co = c_off.numpy()
+        pos = np.concatenate([np.arange(co[i], co[i + 1]) for i in imp])
+        assert np.array_equal(a["scores"], scores.numpy()[pos])
+        assert np.array_equal(a["ranks"], ranks.numpy()[pos].astype(np.float32))
+        if n_imp == 7:
+            assert len(imp) == n_imp
+        else:
+            assert bench.DUMP_MAX_CANDIDATES - 300 < len(pos) <= bench.DUMP_MAX_CANDIDATES
+        assert sum(v.nbytes for v in a.values()) <= 64 << 20
 
 
 def _toy_behaviors():

@@ -1,6 +1,5 @@
 """Pin oracle/oracle.py against outputs of the reference itself (tests/golden,
 minted by oracle/make_golden.py) -- CPU only."""
-import hashlib
 import os
 
 import numpy as np
@@ -8,15 +7,8 @@ import pytest
 import torch
 
 from oracle import oracle
+from oracle.make_golden import sd_digest
 from news_recommendation_project_v2_b200 import synthetic as syn
-
-
-def _digest(sd):
-    h = hashlib.sha256()
-    for k in sorted(sd):
-        h.update(k.encode())
-        h.update(sd[k].detach().contiguous().numpy().tobytes())
-    return h.hexdigest()
 
 
 def _load(golden_dir, name):
@@ -28,7 +20,7 @@ def test_latent_pool_matches_reference(golden_dir, name):
     g = _load(golden_dir, name)
     dim, L, B, S, seed = (int(g[k]) for k in ("dim", "L", "B", "S", "seed"))
     sd = syn.make_latent_state_dict(dim, L, seed=seed)
-    assert _digest(sd) == str(g["sd_sha256"]), "weight generator drifted from the golden run"
+    assert sd_digest(sd) == str(g["sd_sha256"]), "weight generator drifted from the golden run"
     assert sorted(sd.keys()) == list(g["keys"])
     x, mask = syn.make_token_batch(B, S, dim, seed=seed + 1)
     pooled = oracle.latent_pool(sd, x, mask, dtype=torch.float64).float().numpy()
@@ -59,7 +51,7 @@ def test_final_attention_score_rank_matches_reference(golden_dir, name):
     g = _load(golden_dir, name)
     dim, hidden, n_rows, n_imp, seed = (int(g[k]) for k in ("dim", "hidden", "n_rows", "n_imp", "seed"))
     sd = syn.make_final_attention_state_dict(dim, hidden, seed=seed)
-    assert _digest(sd) == str(g["sd_sha256"])
+    assert sd_digest(sd) == str(g["sd_sha256"])
     table = syn.make_table(n_rows, dim, seed=seed + 2)
     imp = syn.make_impressions(n_imp, n_rows, h_max=50, cand=str(g["cand"]), seed=seed + 3)
     out = oracle.final_second_attention_score(sd, table, imp.hist_idx, imp.hist_len, imp.cand_idx, imp.cand_len,
@@ -86,7 +78,7 @@ def test_final_attention_medium_fixture_matches_reference(golden_dir):
     g = _load(golden_dir, "final_medium_d1024")
     dim, hidden, n_rows, n_imp, seed = (int(g[k]) for k in ("dim", "hidden", "n_rows", "n_imp", "seed"))
     sd = syn.make_final_attention_state_dict(dim, hidden, seed=seed)
-    assert _digest(sd) == str(g["sd_sha256"])
+    assert sd_digest(sd) == str(g["sd_sha256"])
     table = syn.make_table(n_rows, dim, seed=seed + 2)
     imp = syn.make_impressions(n_imp, n_rows, h_max=50, cand=str(g["cand"]), seed=seed + 3)
     ref_ranks = g["ranks"].astype(np.float64)
@@ -111,7 +103,7 @@ def test_latent_user_encoder_long_history_matches_reference(golden_dir):
     g = _load(golden_dir, "latent_user_cfg5_d1024_L1024_H200")
     dim, L, n_rows, n_imp, h_max, seed = (int(g[k]) for k in ("dim", "L", "n_rows", "n_imp", "h_max", "seed"))
     sd = syn.make_latent_state_dict(dim, L, seed=seed)
-    assert _digest(sd) == str(g["sd_sha256"])
+    assert sd_digest(sd) == str(g["sd_sha256"])
     table = syn.make_table(n_rows, dim, seed=seed + 2)
     imp = syn.make_long_history_impressions(n_imp, n_rows, h_max, seed + 3)
     assert np.array_equal(imp.hist_len, g["hist_len"]) and int(imp.hist_len.max()) == h_max == 200
