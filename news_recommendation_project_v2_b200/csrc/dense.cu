@@ -20,9 +20,10 @@ __device__ __forceinline__ void store_elem(void* p, int dt, int64_t i, float v) 
     reinterpret_cast<__nv_bfloat16*>(p)[i] = __float2bfloat16_rn(v);
 }
 
-// One warp per row.  Two-pass mean / variance in fp32 like ATen's LayerNorm; the row is re-read
-// from L1 rather than cached so that any `dim` works.  Optionally gathers the source row through
-// `row_map` (varlen token packing) and emits an fp32 copy of the raw row (the residual operand).
+// One warp per row.  Two-pass mean / variance in fp32 of x - x0 (x0 = the row's first element, see
+// layer_norm_vec_kernel); the row is re-read from L1 rather than cached so that any `dim` works.
+// Optionally gathers the source row through `row_map` (varlen token packing) and emits an fp32 copy
+// of the raw row (the residual operand).
 __global__ void __launch_bounds__(256)
 layer_norm_kernel(const void* x, int x_dtype, int64_t ldx, const int32_t* row_map, const float* gamma,
                   const float* beta, void* y, int y_dtype, int64_t ldy, float* copy_f32, int64_t ldcopy,
@@ -34,18 +35,19 @@ layer_norm_kernel(const void* x, int x_dtype, int64_t ldx, const int32_t* row_ma
   for (int64_t r = warp_id; r < n; r += n_warps) {
     const int64_t src = row_map != nullptr ? (int64_t)row_map[r] : r;
     const int64_t xo = src * ldx;
+    const float x0 = load_elem(x, x_dtype, xo);  // shift of the statistics (see layer_norm_vec_kernel)
     float s = 0.f;
-    for (int i = lane; i < dim; i += 32) s += load_elem(x, x_dtype, xo + i);
-    const float mean = warp_sum(s) / (float)dim;
+    for (int i = lane; i < dim; i += 32) s += load_elem(x, x_dtype, xo + i) - x0;
+    const float mean = warp_sum(s) / (float)dim;  // of x - x0
     float q = 0.f;
     for (int i = lane; i < dim; i += 32) {
-      const float d = load_elem(x, x_dtype, xo + i) - mean;
+      const float d = (load_elem(x, x_dtype, xo + i) - x0) - mean;
       q = fmaf(d, d, q);
     }
     const float rstd = rsqrtf(warp_sum(q) / (float)dim + eps);
     for (int i = lane; i < dim; i += 32) {
       const float v = load_elem(x, x_dtype, xo + i);
-      store_elem(y, y_dtype, r * ldy + i, (v - mean) * rstd * gamma[i] + beta[i]);
+      store_elem(y, y_dtype, r * ldy + i, ((v - x0) - mean) * rstd * gamma[i] + beta[i]);
       if (copy_f32 != nullptr) copy_f32[r * ldcopy + i] = v;
     }
   }
@@ -71,21 +73,27 @@ layer_norm_vec_kernel(const void* x, int64_t ldx, const int32_t* row_map, const 
     if (r + n_warps < n) src_next = row_map != nullptr ? (int64_t)row_map[r + n_warps] : r + n_warps;
     const char* base = reinterpret_cast<const char*>(xin + src * ldx);
     float v[NV][EPV];
-    float s = 0.f;
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
       const uint4 u = *reinterpret_cast<const uint4*>(base + (size_t)(lane + 32 * i) * 16);
       Vec16<TIN>::unpack(u, v[i]);
-#pragma unroll
-      for (int k = 0; k < EPV; ++k) s += v[i][k];
     }
-    const float mean = warp_sum(s) / (float)dim;
+    // Statistics of x - x0, x0 = the row's first element: sum(x) / dim rounds the mean by up to an ulp of x, and
+    // (x - mean) * rsqrt(var + eps) turns that into O(1) when the spread is far below the magnitude -- a constant
+    // row with eps 1e-12 came out as beta +- 0.4 gamma.  x - x0 is exact there, so the mean and every deviation are.
+    const float x0 = __shfl_sync(kFullMask, v[0][0], 0);
+    float s = 0.f;
+#pragma unroll
+    for (int i = 0; i < NV; ++i)
+#pragma unroll
+      for (int k = 0; k < EPV; ++k) s += v[i][k] - x0;
+    const float mean = warp_sum(s) / (float)dim;  // of x - x0
     float q = 0.f;
 #pragma unroll
     for (int i = 0; i < NV; ++i)
 #pragma unroll
       for (int k = 0; k < EPV; ++k) {
-        const float d = v[i][k] - mean;
+        const float d = (v[i][k] - x0) - mean;
         q = fmaf(d, d, q);
       }
     const float rstd = rsqrtf(warp_sum(q) / (float)dim + eps);
@@ -97,10 +105,10 @@ layer_norm_vec_kernel(const void* x, int64_t ldx, const int32_t* row_map, const 
       for (int k = 0; k < EPV; k += 4) {
         const float4 g4 = *reinterpret_cast<const float4*>(gamma + e0 + k);
         const float4 b4 = *reinterpret_cast<const float4*>(beta + e0 + k);
-        o[k] = (v[i][k] - mean) * rstd * g4.x + b4.x;
-        o[k + 1] = (v[i][k + 1] - mean) * rstd * g4.y + b4.y;
-        o[k + 2] = (v[i][k + 2] - mean) * rstd * g4.z + b4.z;
-        o[k + 3] = (v[i][k + 3] - mean) * rstd * g4.w + b4.w;
+        o[k] = ((v[i][k] - x0) - mean) * rstd * g4.x + b4.x;
+        o[k + 1] = ((v[i][k + 1] - x0) - mean) * rstd * g4.y + b4.y;
+        o[k + 2] = ((v[i][k + 2] - x0) - mean) * rstd * g4.z + b4.z;
+        o[k + 3] = ((v[i][k + 3] - x0) - mean) * rstd * g4.w + b4.w;
       }
       if (y_dtype == NRB_BF16) {
         __nv_bfloat16* yo = reinterpret_cast<__nv_bfloat16*>(y) + r * ldy + e0;

@@ -218,3 +218,58 @@ def test_packed_all_empty_items_give_nan():
     assert torch.isnan(out[[0, 2, 4]]).all() and torch.isfinite(out[[1, 3]]).all()
     want = m.forward_packed(tok.cuda(), torch.tensor([0, 4, 10])).cpu()
     assert torch.equal(out[[1, 3]], want)
+
+
+def _softmax_gemm_tiles_per_cluster(n_tokens, heads, latents_padded):
+    """Tiles per persistent cluster of the fused softmax GEMM over n_tokens rows, the way launch_gemm sizes its grid
+    (clusters of Lp / 256 CTAs share a 128-row block; at most SMs / cluster co-resident clusters)."""
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    cs = max(1, latents_padded // 256)
+    units = -(-n_tokens // 128) * (heads * latents_padded // 256 // cs)
+    return units / (sms // cs)
+
+
+def _token_batch_with_at_least(n_valid, S, dim, seed):
+    """Padded token batch [B, S, dim] (prefix masks, 1..S tokens per item) holding at least n_valid tokens."""
+    g = torch.Generator().manual_seed(seed)
+    lens = torch.randint(1, S + 1, (2 * n_valid // S + 2 * S,), generator=g)
+    B = int(torch.searchsorted(torch.cumsum(lens, 0), n_valid).item()) + 1
+    lens = lens[:B]
+    mask = (torch.arange(S)[None, :] < lens[:, None]).to(torch.int32)
+    return torch.randn(B, S, dim, generator=g), mask
+
+
+def test_latent_stage_a_several_tiles_per_cta():
+    """Stage A at scale (bf16, fused softmax GEMM with one 256-column tile per row block): enough valid tokens that
+    every CTA works through >= 3 tiles with the device-side row count and row map of the masked path, and more than
+    1,024 items in one chunk (the carry of the item-offset scan).  Padded + masked and packed forms against the fp64
+    oracle on the device, and bit-equal to each other."""
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    m = _model(256, 64, 31, "bf16", heads=4, dim_head=64)
+    x, mask = _token_batch_with_at_least(3 * sms * 128 + 200, 20, 256, seed=32)
+    n_tok = int(mask.sum())
+    assert _softmax_gemm_tiles_per_cluster(n_tok, 4, 64) >= 3 and mask.shape[0] > 1024
+    from news_recommendation_project_v2_b200 import config
+    assert x.shape[0] * x.shape[1] <= config.LATENT_MAX_TOKENS  # one chunk
+    sd = {k: v.cuda() for k, v in m.state_dict().items()}
+    want = oracle.latent_pool(sd, x.cuda(), mask.cuda(), heads=4, dim_head=64, dtype=torch.float64)
+    got = m(x.cuda(), mask.cuda())
+    torch.testing.assert_close(got.double(), want, atol=TOL["bf16"], rtol=0)
+    off = torch.zeros(mask.shape[0] + 1, dtype=torch.int64)
+    off[1:] = torch.cumsum(mask.sum(1), 0)
+    packed = m.forward_packed(x[mask.bool()].cuda(), off)
+    assert torch.equal(packed, got)
+
+
+def test_latent_cluster_of_4_several_tiles_per_cluster():
+    """d=1024, L=1024 (8 heads x 512): the softmax over 1,024 latents spans a cluster of 4 CTAs; enough tokens that
+    each co-resident cluster works through >= 3 row blocks (the statistics barrier on a cluster's later tiles)."""
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    m = _model(1024, 1024, 41, "bf16")
+    need = -(-3 * (sms // 4) // 8) * 128  # 8 units per 128-row block
+    x, mask = _token_batch_with_at_least(need + 200, 24, 1024, seed=42)
+    assert _softmax_gemm_tiles_per_cluster(int(mask.sum()), 8, 1024) >= 3
+    sd = {k: v.cuda() for k, v in m.state_dict().items()}
+    want = oracle.latent_pool(sd, x.cuda(), mask.cuda(), heads=8, dim_head=512, dtype=torch.float64)
+    got = m(x.cuda(), mask.cuda())
+    torch.testing.assert_close(got.double(), want, atol=TOL["bf16"], rtol=0)

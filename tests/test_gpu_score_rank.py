@@ -84,23 +84,42 @@ def _oracle_pool_score(X, E, T, imp, mode):
     return users, scores.numpy()
 
 
+# every (dtype, vectors per lane) instantiation: NV = dim * elemsize / 512 = 1..8
 @pytest.mark.parametrize("dtype,dim", [(torch.float32, 768), (torch.bfloat16, 768), (torch.bfloat16, 1024),
-                                       (torch.float32, 1024), (torch.bfloat16, 256), (torch.float32, 128)])
-@pytest.mark.parametrize("mode", [0, 1])
-def test_score_rank_vs_oracle(ops, dtype, dim, mode):
+                                       (torch.float32, 1024), (torch.bfloat16, 256), (torch.float32, 128)] +
+                         [(torch.bfloat16, d) for d in (512, 1280, 1536, 1792, 2048)] +
+                         [(torch.float32, d) for d in (256, 384, 512, 640, 896)])
+@pytest.mark.parametrize("mode,blend", [(0, False), (1, False), (0, True)], ids=["0", "1", "0-blend"])
+def test_score_rank_vs_oracle(ops, dtype, dim, mode, blend):
     n_rows, n_imp = 3000, 257
     g = torch.Generator().manual_seed(11)
     T = syn.make_table(n_rows, dim, seed=5).to(dtype)
     X = torch.randn(n_rows, dim, generator=g).to(dtype)
     E = torch.exp(0.5 * torch.randn(n_rows, dim, generator=g)).to(dtype) if mode == 0 else None
     imp = syn.make_impressions(n_imp, n_rows, h_max=50, cand="large", seed=17)
-    imp.cand_len[3] = 600  # above the in-smem rank capacity
-    imp.cand_idx = np.random.default_rng(1).integers(0, n_rows, size=int(imp.cand_len.sum())).astype(np.int32)
+    rng = np.random.default_rng(1)
+    # candidate counts around the in-smem rank capacity (512) and above it
+    imp.cand_len[3:7] = [600, 511, 512, 513]
+    imp.cand_idx = rng.integers(0, n_rows, size=int(imp.cand_len.sum())).astype(np.int32)
+    # history lengths at the edges of the kernel's load batches (HR rows in flight) and of its 32-row blocks
+    nv = dim * T.element_size() // 512
+    hr = max(1, 16 // (nv * (2 if mode == 0 else 1)))
+    imp.hist_len[10:17] = [1, hr, hr + 1, 32, 33, 64, 65]
+    if blend:
+        imp.hist_len[20:22] = 0  # no history: the baseline alone
+    imp.hist_idx = rng.integers(0, n_rows, size=int(imp.hist_len.sum())).astype(np.int32)
+    base = torch.randn(n_rows, generator=g) if blend else None
+    alpha = 0.7 if blend else 1.0
     n_c = int(imp.cand_len.sum())
     user, scores, ranks = ops.score_rank(
         mode, X.cuda(), None if E is None else E.cuda(), T.cuda(), torch.from_numpy(imp.hist_idx).cuda(),
-        _csr(imp.hist_len), torch.from_numpy(imp.cand_idx).cuda(), _csr(imp.cand_len), n_c, want_user=True)
+        _csr(imp.hist_len), torch.from_numpy(imp.cand_idx).cuda(), _csr(imp.cand_len), n_c, want_user=True,
+        cand_base=None if base is None else base.cuda(), blend_alpha=alpha)
     want_u, want_s = _oracle_pool_score(X, E, T, imp, mode)
+    if blend:  # alpha * cos + (1 - alpha) * base; impressions without history get the base alone
+        b = base.double().numpy()[imp.cand_idx]
+        has_hist = np.repeat(imp.hist_len > 0, imp.cand_len)
+        want_s = np.where(has_hist, alpha * want_s + (1 - alpha) * b, b)
     # fp32 accumulation of <= 50 rows / dot products of length d: 1e-5 abs on O(1) values
     np.testing.assert_allclose(user.cpu().numpy(), want_u.float().numpy(), atol=2e-5, rtol=2e-5)
     np.testing.assert_allclose(scores.cpu().numpy(), want_s, atol=5e-6, rtol=0)
