@@ -51,6 +51,7 @@ extern "C" {
 #define NRB_EPI_RESIDUAL 3  /* y = acc + bias + res                   latent_attention.py:162-163 */
 #define NRB_EPI_GEGLU 4     /* y[j] = a_j * gelu_erf(g_j), W rows interleaved in pairs (a0,a1,g0,g1,a2,a3,g2,g3..) latent_attention.py:24-27 */
 #define NRB_EPI_SOFTMAX 5   /* y = softmax over each group of `group` columns (first `group_valid` valid); latent_attention.py:69-72 */
+#define NRB_EPI_TOPK 6      /* internal to nrb_recommend: per-row top-k of acc * scale[col], no output tile */
 
 typedef void* nrb_stream_t;
 
@@ -234,6 +235,32 @@ int nrb_latent_forward_packed(const nrb_latent_weights* w, const void* x_packed,
                               int64_t n_tokens, const int32_t* item_off, int64_t batch,
                               float* pooled_out, void* workspace, size_t workspace_bytes,
                               nrb_stream_t stream);
+
+/* ---- whole-table retrieval: the k best rows of the table for each user -------------------------------------
+ * (no reference counterpart: the reference only scores candidate lists it is given.)
+ *   score(u, r) = (u / max(|u|, 1e-8)) . c_r / max(|c_r|, 1e-8)    -- the cosine of nrb_score_rank
+ * out_rows int32 [n_users, k] / out_scores fp32 [n_users, k]: score descending, equal scores by ascending row id
+ * (-0.0 equals 0.0), NaN scores never returned, (-1, NaN) where a user has fewer than k eligible rows.
+ *   precision NRB_BF16: `table` and `table_op` are the bf16 table (the same pointer); users are normalised in fp32
+ *                       and rounded to bf16.
+ *   precision NRB_F32 : `table` is the fp32 table (row norms), `table_op` its nrb_split_rows(role 1) copy [n_rows,
+ *                       3*dim]; users are split with role 0, so ONE tensor-core GEMM over K' = 3*dim scores at ~2^-17
+ *                       relative.  The FFMA GEMM has no top-k epilogue.
+ *   users           : fp32 [n_users, dim] (e.g. nrb_score_rank's user_out).
+ *   excl_idx / excl_off : optional CSR (int32 ids, int64 offsets [n_users + 1], n_excl = excl_off[n_users] or more)
+ *                     of rows never returned for each user (their history); ids may repeat and need not be sorted.
+ *                     An id outside [0, n_rows) sets bit 0 of *err_flag.  Both NULL: nothing excluded.
+ * The scores are computed by one tcgen05 GEMM whose epilogue keeps each row's running top-k in shared memory: the
+ * [n_users, n_rows] score matrix never exists in memory.  A user's result does not depend on the other users of the
+ * call as long as the same GEMM configuration runs (n_users <= 128: single CTAs; more: CTA pairs).
+ * Limits: 1 <= k <= 32, dim % 64 == 0, any n_users >= 1 and n_rows >= 1.  Invalid arguments are rejected before any
+ * CUDA call (the workspace query then returns 0). */
+size_t nrb_recommend_workspace_bytes(int precision, int dim, int64_t n_rows, int64_t n_users, int64_t n_excl, int k);
+int nrb_recommend(int precision, int dim, int64_t n_rows, const void* table, int64_t table_stride,
+                  const void* table_op, int64_t op_stride, const float* users, int64_t users_stride, int64_t n_users,
+                  const int32_t* excl_idx, const int64_t* excl_off, int64_t n_excl, int k,
+                  int32_t* out_rows, float* out_scores, int32_t* err_flag, void* workspace, size_t workspace_bytes,
+                  nrb_stream_t stream);
 
 /* ---- MIND metrics on device (consumer of the ranks; "next" row of the hot path) ---------------
  * replaces evaluation.py:34-98 (score_row per impression in a 4-process pool + mean):

@@ -17,6 +17,7 @@ LIB_PATH = os.environ.get("NRB200_LIB") or os.path.join(_PKG, "libnrb200.so")  #
 F32, BF16 = 0, 1
 POOL_FINAL_ATTENTION, POOL_MEAN_L2 = 0, 1
 EPI_NONE, EPI_RELU, EPI_EXP, EPI_RESIDUAL, EPI_GEGLU, EPI_SOFTMAX = 0, 1, 2, 3, 4, 5
+RECOMMEND_MAX_K = 32  # longest list nrb_recommend returns per user
 
 _c_void_p, _i64, _i32, _f32, _sz = C.c_void_p, C.c_int64, C.c_int, C.c_float, C.c_size_t
 
@@ -93,6 +94,10 @@ PROTOTYPES = {
                                          _c_void_p, _c_void_p, _sz, _c_void_p]),
     "nrb_latent_forward": (_i32, [C.POINTER(LatentWeights), _c_void_p, _i32, _i64, _i32, _c_void_p,
                                   _c_void_p, _c_void_p, _c_void_p, _sz, _i64, C.POINTER(_i64), _c_void_p]),
+    "nrb_recommend_workspace_bytes": (_sz, [_i32, _i32, _i64, _i64, _i64, _i32]),
+    "nrb_recommend": (_i32, [_i32, _i32, _i64, _c_void_p, _i64, _c_void_p, _i64, _c_void_p, _i64, _i64,
+                             _c_void_p, _c_void_p, _i64, _i32, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _sz,
+                             _c_void_p]),
 }
 
 _lock = threading.Lock()

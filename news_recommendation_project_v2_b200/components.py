@@ -4,6 +4,7 @@
   SaveEmbeddingComponent     components.py:178-222  table writer  (`<dataset>.pt`, `query_<dataset>.pt`)
   LoadEmbeddingComponent     components.py:225-258  table reader
   FinalAttentionComponent    components.py:980-1027 gather + user encoder + cosine + dense rank
+  TopKRecommendationComponent (new)                 the k best news of the whole table per user
 
 Only `transform` is in scope (scripts/eval.py's path); training stays with the reference."""
 from __future__ import annotations
@@ -14,7 +15,7 @@ from typing import Any, Optional
 import numpy as np
 import torch
 
-from .data_model_helper import get_final_second_attention_score
+from .data_model_helper import get_final_second_attention_score, get_top_k_recommendations
 from .data_utils import split_impressions_and_history
 from .modeling_utils import get_final_attention_model
 from .pipeline import PipelineComponent, check_req_keys
@@ -111,3 +112,35 @@ class FinalAttentionComponent(PipelineComponent):
 
     def train(self, context_dict, val_context_dict=None) -> None:
         raise NotImplementedError("training is out of scope for the B200 hot path (use the reference trainer)")
+
+
+class TopKRecommendationComponent(PipelineComponent):
+    """Recommends, for every user with a history, the k news of the whole table that score best against the user
+    vector (the cosine FinalAttentionComponent ranks candidates by), history excluded by default.  Adds
+    `top_k_rows` (int32 [U, k] row ids), `top_k_scores` (float32 [U, k]) and `top_k_news` (object [U, k] news ids
+    from `news_list`, None where a user has fewer than k eligible news)."""
+
+    required_keys = {"news_embeddings", "history_rev_ind_array", "history_len_list", "news_list"}
+
+    def __init__(self, k: int = 10, attention_model_path: Optional[Path] = None, attention_model=None,
+                 exclude_history: bool = True, precision=None, **_unused):
+        self.k = int(k)
+        self.attention_model = attention_model if attention_model is not None else \
+            get_final_attention_model(attention_model_path)
+        self.exclude_history = exclude_history
+        self.precision = precision
+
+    def transform(self, context_dict: dict[str, Any]) -> dict[str, Any]:
+        check_req_keys(self.required_keys, context_dict)
+        out = context_dict.copy()
+        res = get_top_k_recommendations(
+            out["history_rev_ind_array"][0], out["history_len_list"], out["news_embeddings"], self.attention_model,
+            k=self.k, exclude_history=self.exclude_history, query_news_embeddings=out.get("query_news_embeddings"),
+            precision=self.precision)
+        out.update(res)
+        news = np.asarray(out["news_list"], dtype=object)
+        rows = res["top_k_rows"]
+        top = np.full(rows.shape, None, dtype=object)
+        top[rows >= 0] = news[rows[rows >= 0]]
+        out["top_k_news"] = top
+        return out

@@ -10,6 +10,20 @@ int gemm_bf16_tc(int epi, int out_dtype, const void* a, int64_t lda, const void*
                  const void* res, int64_t ldres, void* y, int64_t ldy, int64_t M, const int* m_dev, int N, int K,
                  int group, int group_valid, cudaStream_t st, int res_dtype = NRB_F32,
                  const int32_t* res_map = nullptr);
+// gemm_tc.cu -- tcgen05 GEMM with the fused top-k epilogue (NRB_EPI_TOPK)
+struct TopkPlan {
+  int cg;              // 1: single CTA (M <= 128), 2: CTA pairs
+  int rows_per_block;  // 128 * cg
+  int64_t m_tiles, n_per_row, units, n_units, slots;
+};
+// CTA (pair) whose contiguous unit range holds unit u: the largest c with floor(c * units / n_units) <= u
+__host__ __device__ inline int64_t topk_owner(const TopkPlan& t, int64_t u) {
+  return ((u + 1) * t.n_units - 1) / t.units;
+}
+TopkPlan topk_plan(int64_t M, int64_t N);
+int gemm_topk_tc(const void* a, int64_t lda, const void* w, int64_t ldw, const float* scale, const int64_t* excl_off,
+                 const int32_t* excl_sorted, int64_t M, int N, int K, int k, const TopkPlan& plan, void* parts,
+                 cudaStream_t st);
 // gemm_simt.cu -- FFMA (fp32 operands)
 int gemm_f32_simt(int epi, int out_dtype, const void* a, int64_t lda, const void* w, int64_t ldw,
                   const float* bias, const void* res, int64_t ldres, void* y, int64_t ldy, int64_t M,

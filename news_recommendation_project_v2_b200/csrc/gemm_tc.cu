@@ -44,16 +44,18 @@ constexpr int kGemmThreads = (kCtrlWarps + kEpiWarps) * 32;
 constexpr int kGroupBytes = kBM * 128;  // one 128-row x 64-column bf16 staging group (swizzle-128B)
 constexpr int kMaxCluster = 4;  // softmax groups up to 4 x 256 = 1024 columns
 constexpr int kSmemLimit = 232448;  // 227 KB opt-in limit per CTA
+constexpr int kTopkMaxK = 32;       // NRB_EPI_TOPK: longest list an epilogue thread keeps (8-byte entries in smem)
 
 template <int BN, int EPI, bool OUT_BF16, int CG = 1>
 struct GemmCfg {
   static_assert(CG == 1 || (CG == 2 && BN == 256 && EPI != NRB_EPI_SOFTMAX), "CTA pairs: 256-wide tiles, no softmax");
   static constexpr bool kStaged = OUT_BF16;
   static constexpr bool kSoftmax = EPI == NRB_EPI_SOFTMAX;
+  static constexpr bool kTopk = EPI == NRB_EPI_TOPK;
   // fp32 outputs: every epilogue warp transposes its 32x32 accumulator chunk through a private 4 KB smem patch so
   // that the residual loads and the output stores touch 4 rows x 128 contiguous bytes per instruction instead of
   // 32 rows x 16 bytes (GEGLU with fp32 output -- unused on the hot path -- keeps the direct row-per-lane stores)
-  static constexpr bool kXpose = !OUT_BF16 && EPI != NRB_EPI_GEGLU;
+  static constexpr bool kXpose = !OUT_BF16 && EPI != NRB_EPI_GEGLU && !kTopk;
   static constexpr int kXposeBytes = kXpose ? kEpiWarps * 4096 : 0;
   static constexpr int kHalves = BN / 128;  // epilogue column halves (128 accumulator columns each)
   static constexpr int kABytes = kBM * kBK * 2;
@@ -61,7 +63,10 @@ struct GemmCfg {
   static constexpr int kStageBytes = kABytes + kBBytes;
   static constexpr int kStagingBytes = kStaged ? kHalves * 2 * kGroupBytes : 0;  // double buffered per half
   static constexpr int kXchgBytes = kSoftmax ? 2 * 2 * (2 * kMaxCluster) * 128 * 4 : 0;  // [parity][m|s][participant][row]
-  static constexpr int kFixedBytes = 1024 /*align*/ + 512 /*barriers*/ + kStagingBytes + kXposeBytes + kXchgBytes;
+  // top-k: one list of kTopkMaxK (score, row) entries per epilogue thread, entry j of thread t at [j][t]
+  static constexpr int kListBytes = kTopk ? kTopkMaxK * kEpiWarps * 32 * 8 : 0;
+  static constexpr int kFixedBytes =
+      1024 /*align*/ + 512 /*barriers*/ + kStagingBytes + kXposeBytes + kXchgBytes + kListBytes;
   static constexpr int kStagesRaw = (kSmemLimit - kFixedBytes) / kStageBytes;
 #ifndef NRB_MAX_STAGES
 #define NRB_MAX_STAGES 6
@@ -71,6 +76,7 @@ struct GemmCfg {
   static constexpr int kSmemBytes = kStages * kStageBytes + kFixedBytes;
   static_assert(kStages >= 2, "pipeline too shallow");
   static_assert(!kSoftmax || OUT_BF16, "softmax epilogue writes bf16 probabilities");
+  static_assert(!kTopk || (!OUT_BF16 && BN == 256), "top-k epilogue: 256-wide tiles, no output tile");
 };
 
 struct GemmParams {
@@ -88,6 +94,13 @@ struct GemmParams {
   int group_valid;  // softmax: valid columns per group (L <= Lp)
   int cluster;      // softmax: CTAs per cluster = max(1, Lp / 256)
   PushJob push;     // rows of an earlier result that the spare warp multicasts to every rank while the GEMM runs
+  // NRB_EPI_TOPK reuses fields (the parameter block of every other instantiation stays as it is):
+  //   bias    = per-column scale 1 / max(|w_n|, 1e-8), NaN from column N up to the next multiple of 256
+  //   res     = int64 CSR offsets [M + 1] of the excluded columns of each row (NULL: nothing excluded)
+  //   res_map = the excluded columns, sorted ascending within each row
+  //   y       = partial lists, 8-byte (score, column) entries [rows][2 halves][ldy slots][group]
+  //   ldy     = slots per (row, half): CTAs (pairs) whose contiguous unit range touches one row block
+  //   group   = k
 };
 
 __device__ __forceinline__ float ex2_approx(float x) {
@@ -257,7 +270,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   uint8_t* staging = smem + kStages * Cfg::kStageBytes;  // [kHalves][2][16 KB], 1024-aligned
   uint8_t* xpose = staging + Cfg::kStagingBytes;                         // [kEpiWarps][4 KB]
   float* xbuf = reinterpret_cast<float*>(xpose + Cfg::kXposeBytes);      // [2][2*kMaxCluster][128]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(xpose + Cfg::kXposeBytes + Cfg::kXchgBytes);
+  uint2* topk_list = reinterpret_cast<uint2*>(xpose + Cfg::kXposeBytes + Cfg::kXchgBytes);  // [kTopkMaxK][256]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(xpose + Cfg::kXposeBytes + Cfg::kXchgBytes + Cfg::kListBytes);
   uint64_t* full_bar = bars;                      // [kStages] TMA -> MMA
   uint64_t* empty_bar = bars + kStages;           // [kStages] MMA -> TMA
   uint64_t* tmem_full = bars + 2 * kStages;       // [2] MMA -> epilogue
@@ -281,6 +295,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   const int n_units_per_row = n_tiles / CS;  // host guarantees n_tiles % CS == 0
   const int64_t total_units = (int64_t)m_tiles * n_units_per_row;
   const int k_blocks = p.K / kBK;
+  // Units are strided over the grid (u = unit, unit + n_units, ...), except for the top-k epilogue: there each unit
+  // takes one contiguous range, row block by row block with N tiles ascending, so that a thread's list lives across
+  // all the tiles its CTA does for one row block and is written out once per (row block, CTA).
+  int64_t u_first = unit, u_last = total_units, u_step = n_units;
+  if constexpr (Cfg::kTopk) {
+    u_first = (int64_t)unit * total_units / n_units;
+    u_last = ((int64_t)unit + 1) * total_units / n_units;
+    u_step = 1;
+  }
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tensormap(&map_a);
@@ -319,7 +342,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
-      for (int64_t u = unit; u < total_units; u += n_units) {
+      for (int64_t u = u_first; u < u_last; u += u_step) {
         const int m_blk = (int)(u / n_units_per_row) * CG + (CG == 2 ? (int)cta_rank : 0);
         const int n_blk = (int)(u % n_units_per_row) * CS + (CG == 2 ? 0 : (int)cta_rank);
         for (int kb = 0; kb < k_blocks; ++kb) {
@@ -357,7 +380,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       uint32_t phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
-      for (int64_t u = unit; u < total_units; u += n_units) {
+      for (int64_t u = u_first; u < u_last; u += u_step) {
         ptx::mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
         ptx::tc_fence_after();
         const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN);
@@ -411,6 +434,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     int acc = 0;
     uint32_t acc_phase = 0;
     uint32_t it = 0;
+    int topk_cnt = 0;            // top-k: entries in this thread's list
+    float topk_thr = -INFINITY;  // top-k: score a column must beat (the k-th best once the list is full)
+    int64_t hcur = 0, hend = 0;  // top-k: cursor into this row's sorted excluded columns
     // accumulator hand-back: the (leader's) MMA warp waits for every epilogue warp of the pair
     auto release_tmem = [&](int a) {
       // (TMEM reads are ordered by tcgen05.fence::before_thread_sync; no memory release is needed, which
@@ -420,7 +446,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       else
         ptx::mbar_arrive(&tmem_empty[a]);
     };
-    for (int64_t u = unit; u < total_units; u += n_units, ++it) {
+    for (int64_t u = u_first; u < u_last; u += u_step, ++it) {
       const int m_blk = (int)(u / n_units_per_row) * CG + (CG == 2 ? (int)cta_rank : 0);
       const int n_blk = (int)(u % n_units_per_row) * CS + (CG == 2 ? 0 : (int)cta_rank);
       ptx::mbar_wait(&tmem_full[acc], acc_phase);
@@ -558,6 +584,86 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             }
             gsel ^= 1;
           }
+        }
+      } else if constexpr (Cfg::kTopk) {
+        // ---------- top-k: score = acc * scale[col]; columns that beat the k-th best enter a smem list ----------
+        const int k = p.group;
+        const int64_t m_u = u / n_units_per_row;  // row block of the unit
+        uint2* const list = topk_list + (e * 32 + lane);
+        constexpr int kLs = kEpiWarps * 32;  // stride between a thread's entries (conflict-free: lane-contiguous)
+        const int32_t* const hist = p.res_map;
+        if (u == u_first || u % n_units_per_row == 0) {  // a row-block segment starts: empty list, cursor to colh
+          topk_cnt = 0;
+          topk_thr = -INFINITY;
+          hcur = hend = 0;
+          if (p.res != nullptr && row_ok) {
+            const int64_t* ho = reinterpret_cast<const int64_t*>(p.res);
+            int64_t lo = ho[row], hi = ho[row + 1];
+            hend = hi;
+            while (lo < hi) {
+              const int64_t mid = (lo + hi) >> 1;
+              if (hist[mid] < colh) lo = mid + 1; else hi = mid;
+            }
+            hcur = lo;
+          }
+        }
+        // Columns reach a thread in ascending order within a segment, so a column that ties the k-th best comes
+        // after it in the (score desc, column asc) order and is rejected by the strict compare; NaN never passes.
+        auto consider = [&](float v, int col) {
+          if (!(v > topk_thr)) return;
+          if (hcur < hend) {  // the cursor only moves forward: one L2 load per excluded column crossed
+            while (hcur < hend && hist[hcur] < col) ++hcur;
+            if (hcur < hend && hist[hcur] == col) return;
+          }
+          v += 0.f;  // -0.0 -> +0.0
+          int pos = topk_cnt < k ? topk_cnt : k - 1;
+          while (pos > 0) {
+            const uint2 prev = list[(pos - 1) * kLs];
+            if (__uint_as_float(prev.x) >= v) break;
+            list[pos * kLs] = prev;
+            --pos;
+          }
+          list[pos * kLs] = make_uint2(__float_as_uint(v), (uint32_t)col);
+          if (topk_cnt < k) ++topk_cnt;
+          if (topk_cnt == k) topk_thr = __uint_as_float(list[(k - 1) * kLs].x);
+        };
+        uint32_t rbuf[2][32];
+        ptx::tmem_ld_32x32(taddr, rbuf[0]);
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          const int col0 = colh + c * 32;
+          ptx::tmem_ld_wait();
+          if (c + 1 < 4) ptx::tmem_ld_32x32(taddr + (uint32_t)((c + 1) * 32), rbuf[(c + 1) & 1]);  // prefetch
+          const uint32_t(&r)[32] = rbuf[c & 1];
+          if (c == 3) {
+            ptx::tc_fence_before();
+            __syncwarp();
+            if (lane == 0) release_tmem(acc);
+          }
+          if (!row_ok || col0 >= p.N) continue;
+          float v[32];
+          bool any = false;
+#pragma unroll
+          for (int j = 0; j < 32; j += 4) {
+            // scale is NaN past column N: the TMA's zero fill there never scores
+            const float4 sc = *reinterpret_cast<const float4*>(p.bias + col0 + j);
+            v[j] = __uint_as_float(r[j]) * sc.x;
+            v[j + 1] = __uint_as_float(r[j + 1]) * sc.y;
+            v[j + 2] = __uint_as_float(r[j + 2]) * sc.z;
+            v[j + 3] = __uint_as_float(r[j + 3]) * sc.w;
+            any |= (v[j] > topk_thr) | (v[j + 1] > topk_thr) | (v[j + 2] > topk_thr) | (v[j + 3] > topk_thr);
+          }
+          if (any) {  // rare once the list is full
+#pragma unroll
+            for (int j = 0; j < 32; ++j) consider(v[j], col0 + j);
+          }
+        }
+        // segment ends (row block changes or the range ends): write the list out, padded with (NaN, -1)
+        if ((u + 1 == u_last || (u + 1) % n_units_per_row == 0) && row_ok) {
+          const int64_t c_first = ((m_u * n_units_per_row + 1) * (int64_t)n_units - 1) / total_units;
+          uint2* dst = reinterpret_cast<uint2*>(p.y) + ((row * 2 + hf) * p.ldy + ((int64_t)unit - c_first)) * k;
+          for (int j = 0; j < k; ++j)
+            dst[j] = j < topk_cnt ? list[j * kLs] : make_uint2(0x7fc00000u, 0xffffffffu);
         }
       } else if constexpr (Cfg::kStaged) {
         // ---------- element-wise epilogue, bf16 output through smem + TMA store ----------
@@ -907,6 +1013,52 @@ int gemm_bf16_tc(int epi, int out_dtype, const void* a, int64_t lda, const void*
   }
   return out_dtype == NRB_BF16 ? dispatch_epi<256, true>(epi, ma, mw, my, p, st)
                                : dispatch_epi<256, false>(epi, ma, mw, my, p, st);
+}
+
+// Schedule of the top-k GEMM, computed the way launch_gemm sizes its grid: `units` scheduling units (one 128-row block,
+// or 256 rows on a CTA pair, times one 256-column tile) split into contiguous ranges over `n_units` CTAs (pairs);
+// `slots` = the most CTAs whose range touches one row block, i.e. the partial lists each (row, half) may get.
+TopkPlan topk_plan(int64_t M, int64_t N) {
+  TopkPlan t;
+  t.cg = M > kBM ? 2 : 1;
+  t.rows_per_block = kBM * t.cg;
+  t.m_tiles = (M + t.rows_per_block - 1) / t.rows_per_block;
+  t.n_per_row = (N + 255) / 256;
+  t.units = t.m_tiles * t.n_per_row;
+  t.n_units = std::min<int64_t>(t.units, sm_count_cached() / t.cg);
+  t.slots = 1;
+  for (int64_t m = 0; m < t.m_tiles; ++m)
+    t.slots = std::max(t.slots, topk_owner(t, (m + 1) * t.n_per_row - 1) - topk_owner(t, m * t.n_per_row) + 1);
+  return t;
+}
+
+// Partial top-k lists of (a[M,K] . w[N,K]^T) * scale[N] per row: see GemmParams for the NRB_EPI_TOPK fields.
+int gemm_topk_tc(const void* a, int64_t lda, const void* w, int64_t ldw, const float* scale, const int64_t* excl_off,
+                 const int32_t* excl_sorted, int64_t M, int N, int K, int k, const TopkPlan& plan, void* parts,
+                 cudaStream_t st) {
+  NRB_REQUIRE(M > 0 && N > 0 && K > 0 && K % kBK == 0, "nrb_recommend: bad GEMM shape");
+  NRB_REQUIRE(k >= 1 && k <= kTopkMaxK, "nrb_recommend: k must be in [1, %d]", kTopkMaxK);
+  CUtensorMap ma, mw;
+  int rc = make_tmap_bf16(&ma, a, M, K, lda, kBM);
+  if (rc != NRB_OK) return rc;
+  rc = make_tmap_bf16(&mw, w, N, K, ldw, plan.cg == 2 ? 128 : 256);
+  if (rc != NRB_OK) return rc;
+  GemmParams p = {};
+  p.M = M;
+  p.m_dev = nullptr;
+  p.N = N;
+  p.K = K;
+  p.bias = scale;
+  p.res = excl_off;
+  p.res_dtype = NRB_F32;
+  p.res_map = excl_sorted;
+  p.y = parts;
+  p.ldy = plan.slots;
+  p.group = k;
+  p.cluster = 1;
+  p.push.n_seg = 0;  // the all-gather rides on the dense row kernels only
+  if (plan.cg == 2) return launch_gemm<256, NRB_EPI_TOPK, false, 2>(ma, mw, ma, p, st);
+  return launch_gemm<256, NRB_EPI_TOPK, false, 1>(ma, mw, ma, p, st);
 }
 
 }  // namespace nrb

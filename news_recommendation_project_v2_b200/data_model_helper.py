@@ -3,6 +3,7 @@
   get_final_attention_eval            data_model_helper.py:112-131
   get_cos_sim_scores                  data_model_helper.py:174-239
   get_final_second_attention_score    data_model_helper.py:416-443
+  get_top_k_recommendations           (new) the k best news of the whole table per user
 
 Same positional signatures and return types (CPU tensors / numpy) as the reference; the work is
 one table upload + one dense row transform (cached per table/weights) + one fused CUDA launch
@@ -60,6 +61,23 @@ def get_final_second_attention_score(history_rev_index: np.ndarray, history_len_
         # (data_model_helper.py:442); reproduce that grouping
         grouped = rank_group_preds(scores_np, imp_len)
     return {"scores": scores_np, "grouped_scores": grouped}
+
+
+def get_top_k_recommendations(history_rev_index: np.ndarray, history_len_list: np.ndarray,
+                              news_embeddings: torch.Tensor, model: torch.nn.Module, k: int = 10,
+                              exclude_history: bool = True, query_news_embeddings: Optional[torch.Tensor] = None,
+                              precision=None) -> dict:
+    """The k news of the whole table that score best against each user (no counterpart in the reference, which only
+    scores the candidate lists of the impressions).  Same user vector and cosine as `get_cos_sim_scores`; with
+    `exclude_history` a user's own history is never recommended.
+
+    Returns numpy {"top_k_rows": int32 [U, k] (row ids = `news_list` positions), "top_k_scores": float32 [U, k]},
+    each list by score descending then row id ascending, -1 / NaN where a user has fewer than k eligible news.
+    1 <= k <= 32."""
+    q = query_news_embeddings if isinstance(query_news_embeddings, torch.Tensor) else None
+    eng = cached_engine(news_embeddings, model, q, precision=precision)
+    rows, scores = eng.recommend(history_rev_index, history_len_list, k, exclude_history=exclude_history)
+    return {"top_k_rows": rows.cpu().numpy(), "top_k_scores": scores.cpu().numpy()}
 
 
 def get_classification_preds(news_embeddings: torch.Tensor, model: torch.nn.Module) -> np.ndarray:

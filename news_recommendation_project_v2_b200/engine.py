@@ -162,6 +162,7 @@ class ScoringEngine:
             self._fa_weights = _final_attention_weights(self.model, self.dtype, dev)
             self._fa_weights_key = fp
         self._padded = None
+        self._split_cand = None
         self.cand = torch.empty(n, d, dtype=self.dtype, device=dev)
         self.hist_x = torch.empty(n, d, dtype=self.dtype, device=dev)
         self.hist_e = torch.empty(n, d, dtype=self.dtype, device=dev)
@@ -306,6 +307,7 @@ class ScoringEngine:
         from .latent_attention import LatentAttentionModel
 
         self._padded = None  # new tables may land at the old addresses: padded kernel copies are rebuilt
+        self._split_cand = None  # likewise the split-bf16 copy of an fp32 table that `recommend` scores against
 
         if isinstance(self.model, NewAttention):
             # LayerNorm chain + exp(linear1): per-row, same exp-weighted pooling as FinalAttention
@@ -370,6 +372,54 @@ class ScoringEngine:
         """Positions of the k best candidates of every impression (int32 [I, k], -1 padded), from device scores."""
         with torch.cuda.device(self.device):
             return ops.topk_order(scores_d, cand_off_d, k)
+
+    # -- whole-table retrieval ---------------------------------------------------------------------------------
+    def _table_operand(self) -> torch.Tensor:
+        """The bf16 GEMM operand `recommend` scores against: the table itself for bf16 engines, its [hi|lo|hi]
+        split copy (cached until the tables are rebuilt) for fp32 / fp32x3 engines."""
+        if self.cand.dtype == torch.bfloat16:
+            return self.cand
+        key = (self.cand.data_ptr(), self.cand._version)
+        hit = getattr(self, "_split_cand", None)
+        if hit is None or hit[0] != key:
+            hit = (key, ops.split_rows(self.cand, 1))
+            self._split_cand = hit
+        return hit[1]
+
+    def recommend_device(self, hist_idx_d: torch.Tensor, hist_off_d: torch.Tensor, k: int,
+                         exclude_history: bool = True, err_flag: Optional[torch.Tensor] = None):
+        """Device CSR history (int32 ids, int64 offsets [U + 1]) in, the k best table rows per user out:
+        (rows int32 [U, k], scores fp32 [U, k]) on the device, see `ops.recommend` for the order and padding.
+
+        The user vector is the one `score` pools; its score against row r is the cosine `score` would give r as a
+        candidate.  With `exclude_history` a user's own history rows are never returned.  fp32 and fp32x3 engines
+        score on split-bf16 tensor-core operands (the FFMA GEMM has no top-k epilogue)."""
+        ops._recommend_args(self.dim, k)
+        with torch.cuda.device(self.device):
+            flag = err_flag if err_flag is not None else ops.new_err_flag(self.device)
+            n_imp = hist_off_d.numel() - 1
+            zeros = torch.zeros(n_imp + 1, dtype=torch.int64, device=self.device)
+            empty = torch.zeros(1, dtype=torch.int32, device=self.device)
+            k_x, k_e, k_c = self._kernel_tables()
+            user, _, _ = ops.score_rank(self.pool_mode, k_x, k_e, k_c, hist_idx_d, hist_off_d, empty, zeros, 0,
+                                        want_user=True, want_ranks=False, err_flag=flag)
+            if user.shape[1] != self.dim:
+                user = user[:, :self.dim].contiguous()  # drop the kernel's zero padding: logical rows and width
+            excl = (hist_idx_d, hist_off_d) if exclude_history else (None, None)
+            rows, scores = ops.recommend(self.cand, user, k, table_op=self._table_operand(), excl_idx=excl[0],
+                                         excl_off=excl[1], err_flag=flag)
+            if err_flag is None:
+                ops.raise_on_index_error(flag, "recommend")
+            return rows, scores
+
+    def recommend(self, hist_idx, hist_len, k: int, exclude_history: bool = True):
+        """Host history arrays (`history_rev_ind_array[0]`, `history_len_list`) in: the k best rows of the whole
+        table for each user, (rows int32 [U, k], scores fp32 [U, k]) on the device."""
+        ops._recommend_args(self.dim, k)
+        with torch.cuda.device(self.device):
+            h_off, n_h = _offsets(hist_len, self.device)
+            assert n_h == len(hist_idx), "history index length should match history_len_list"
+            return self.recommend_device(_as_i32(hist_idx, self.device), h_off, k, exclude_history=exclude_history)
 
     def user_vectors(self, hist_idx, hist_len) -> torch.Tensor:
         """get_final_attention_eval: fp32 [I, d] user vectors (device)."""

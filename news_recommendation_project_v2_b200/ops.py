@@ -197,6 +197,63 @@ def score_rank(pool_mode: int, hist_x: torch.Tensor, hist_e: Optional[torch.Tens
     return user, scores, ranks
 
 
+def _recommend_args(dim: int, k: int) -> None:
+    """The limits of nrb_recommend, checked before anything touches a device."""
+    if not 1 <= int(k) <= _lib.RECOMMEND_MAX_K:
+        raise _lib.NrbError(f"recommend: k must be in [1, {_lib.RECOMMEND_MAX_K}] (got {k})")
+    if dim <= 0 or dim % 64:
+        raise _lib.NrbError(f"recommend: the embedding width must be a multiple of 64 (got {dim})")
+
+
+def recommend(table: torch.Tensor, users: torch.Tensor, k: int, table_op: Optional[torch.Tensor] = None,
+              excl_idx: Optional[torch.Tensor] = None, excl_off: Optional[torch.Tensor] = None,
+              err_flag: Optional[torch.Tensor] = None):
+    """The k best rows of the whole table for each user (nrb_recommend): (rows int32 [U, k], scores fp32 [U, k]).
+
+    score = cosine(user, row), ordered by score descending then row id ascending, (-1, NaN) once a user has no
+    eligible rows left.  bf16 tables run the tensor-core GEMM on bf16 operands; fp32 tables run it on split-bf16
+    operands (`table_op` = split_rows(table, 1), built here if not given).  The fp32 FFMA GEMM has no top-k epilogue,
+    so fp32 retrieval always uses the split tensor-core path.  `excl_idx` / `excl_off` (int32 ids, int64 offsets
+    [U + 1]): rows never returned for each user; an out-of-range id raises IndexError (or sets bit 0 of `err_flag`)."""
+    _recommend_args(table.shape[1] if table.dim() == 2 else 0, k)
+    dev = require_device(table.device)
+    _dev(table, "table")
+    _dev(users, "users", torch.float32)
+    n_rows, dim = table.shape
+    if users.dim() != 2 or users.shape[1] != dim:
+        raise _lib.NrbError(f"users must be [U, {dim}]")
+    prec = dtype_code(table.dtype)
+    if table_op is None:
+        table_op = table if prec == BF16 else split_rows(table, 1)
+    _dev(table_op, "table_op", torch.bfloat16)
+    if (excl_idx is None) != (excl_off is None):
+        raise _lib.NrbError("excl_idx and excl_off go together")
+    n_excl = 0
+    if excl_idx is not None:
+        _dev(excl_idx, "excl_idx", torch.int32)
+        _dev(excl_off, "excl_off", torch.int64)
+        if excl_off.numel() != users.shape[0] + 1:
+            raise _lib.NrbError("excl_off must have U + 1 entries")
+        n_excl = excl_idx.numel()
+    U = users.shape[0]
+    rows = torch.empty(U, k, dtype=torch.int32, device=dev)
+    scores = torch.empty(U, k, dtype=torch.float32, device=dev)
+    if U == 0:
+        return rows, scores
+    lib = load()
+    ws_bytes = lib.nrb_recommend_workspace_bytes(prec, dim, n_rows, U, n_excl, int(k))
+    if ws_bytes == 0:
+        check(-1, "nrb_recommend_workspace_bytes")
+    ws = _workspace(dev, ws_bytes, "recommend")
+    flag = err_flag if err_flag is not None else new_err_flag(dev)
+    check(lib.nrb_recommend(prec, dim, n_rows, ptr(table), table.stride(0), ptr(table_op), table_op.stride(0),
+                            ptr(users), users.stride(0), U, ptr(excl_idx), ptr(excl_off), n_excl, int(k), ptr(rows),
+                            ptr(scores), ptr(flag), ptr(ws), ws.numel(), stream_ptr()), "nrb_recommend")
+    if err_flag is None:
+        raise_on_index_error(flag, "recommend")
+    return rows, scores
+
+
 def linear(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None, epilogue: int = _lib.EPI_NONE,
            res: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None, group: int = 0,
            group_valid: int = 0) -> torch.Tensor:
