@@ -105,6 +105,22 @@ struct ScoreRankParams {
   int32_t* err_flag;
 };
 
+// Rows a warp will gather in its next load batches are requested into L2 ahead of time by the lanes that hold their
+// indices (one bulk prefetch per row: no registers, no shared memory, no completion to wait for).  Without it a warp's
+// DRAM requests stop while it computes on a batch it has received; with it the next batches are already on their way
+// and are then read from L2.  Results do not depend on it.  Up to 148 SMs x 16 warps x kPrefetchBatches x 8 KB stay
+// in L2 at a time (19 MB per batch of distance).  Same-box alternating A/B on one B200 (1,000 W), bench headline, bf16
+// d=1024 FinalAttention: kernel 64.1 -> 59.6 ms at a distance of one batch, 60.3 at two, 60.7 at four
+// (profiles/score_prefetch_ab_b200.txt).
+#ifndef NRB_SCORE_PREFETCH
+#define NRB_SCORE_PREFETCH 1
+#endif
+constexpr int kPrefetchBatches = NRB_SCORE_PREFETCH;
+
+__device__ __forceinline__ void prefetch_row_l2(const char* row, int bytes) {
+  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(row), "r"(bytes) : "memory");
+}
+
 template <typename T, int NV>
 __device__ __forceinline__ void load_row(const char* base, int lane, uint4 (&v)[NV]) {
 #pragma unroll
@@ -153,6 +169,12 @@ score_rank_kernel(const ScoreRankParams p) {
         }
       }
       for (int s = 0; s < cnt; s += HR) {
+        // rows of the next kPrefetchBatches batches of this chunk -> L2 (see prefetch_row_l2)
+        if (lane >= s + HR && lane < min(s + HR * (kPrefetchBatches + 1), cnt) &&
+            (s == 0 || lane >= s + HR * kPrefetchBatches)) {
+          prefetch_row_l2(p.hist_x + (int64_t)my * p.hist_stride_bytes, NV * 512);
+          if (MODE == NRB_POOL_FINAL_ATTENTION) prefetch_row_l2(p.hist_e + (int64_t)my * p.hist_stride_bytes, NV * 512);
+        }
         uint4 x[HR][NV];
         uint4 e[MODE == NRB_POOL_FINAL_ATTENTION ? HR : 1][NV];
 #pragma unroll
@@ -249,6 +271,9 @@ score_rank_kernel(const ScoreRankParams p) {
       float my_dot = 0.f, my_sq = 0.f;
       constexpr int CR = (16 / NV) > 0 ? (16 / NV) : 1;  // candidate rows in flight per iteration
       for (int s = 0; s < cnt; s += CR) {
+        if (lane >= s + CR && lane < min(s + CR * (kPrefetchBatches + 1), cnt) &&
+            (s == 0 || lane >= s + CR * kPrefetchBatches))
+          prefetch_row_l2(p.cand + (int64_t)my * p.cand_stride_bytes, NV * 512);
         uint4 a[CR][NV];
 #pragma unroll
         for (int q = 0; q < CR; ++q) {
