@@ -484,7 +484,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 #pragma unroll
           for (int j = 4; j < 32; ++j) m4[j & 3] = fmaxf(m4[j & 3], xv[j]);
           const float m = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3]));
-          const float mb = (m == -INFINITY ? 0.f : m) * kLog2e;  // an all-masked chunk contributes nothing
+          // A chunk with no valid column (only when lp >= 64) exponentiates from 0 here, which gives exp(-inf) = 0,
+          // and keeps -inf as its pass-B scale: 2^(0 - M log2e) would overflow to +inf once the group max M is below
+          // about -88.7, and 0 * inf is NaN.
+          const float mb = (m == -INFINITY ? 0.f : m) * kLog2e;
           f32x2 s2[2] = {splat2(0.f), splat2(0.f)};  // 4 independent chains, two per packed register
           const f32x2 l2e = splat2(kLog2e), nmb = splat2(-mb);
           uint32_t ev[32];
@@ -503,7 +506,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           // exp(x - m_c) replaces the logit IN TMEM: pass B only rescales, so each element costs one ex2
           ptx::tmem_st_32x32(taddr + (uint32_t)(c * 32), ev);
           mx[c] = m;
-          mcb[c] = mb;
+          mcb[c] = m == -INFINITY ? -INFINITY : mb;
           sm[c] = (s4[0] + s4[1]) + (s4[2] + s4[3]);
         }
         ptx::tmem_st_wait();
@@ -563,7 +566,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             __syncwarp();
             if (lane == 0) release_tmem(acc);
           }
-          // p = exp(x - m_c) * 2^((m_c - M) log2e) / S   (masked columns already hold exp(-inf) = 0)
+          // p = exp(x - m_c) * 2^((m_c - M) log2e) / S   (masked columns already hold exp(-inf) = 0; a chunk with
+          // no valid column has m_c = -inf, so its factor is 2^-inf = 0)
           const float f = ex2_approx(mcb[c] - mx[c] * kLog2e) / sm[c];
           float v[32];
           const f32x2 f2 = splat2(f);

@@ -155,17 +155,21 @@ static int pad_latents(int L) {
   return p;
 }
 
+// latent rows of the fold's FFMA GEMMs: the B fold has N = latents, and that GEMM takes N in multiples of 4; the rows
+// past L are zero, so they give zero rows of A and zero columns of B (L4 <= Lp)
+static int fold_latents(int L) { return (L + 3) / 4 * 4; }
+
 struct FoldWs {
   float *cn, *kv, *wqT, *a32, *b32;
   size_t bytes;
 };
 static FoldWs fold_ws(void* base, int dim, int heads, int dim_head, int L) {
   const int inner = heads * dim_head;
-  const int Lp = pad_latents(L);
+  const int Lp = pad_latents(L), L4 = fold_latents(L);
   Workspace ws(base, (size_t)-1);
   FoldWs f;
-  f.cn = (float*)ws.take((size_t)L * dim * 4);
-  f.kv = (float*)ws.take((size_t)L * 2 * inner * 4);
+  f.cn = (float*)ws.take((size_t)L4 * dim * 4);
+  f.kv = (float*)ws.take((size_t)L4 * 2 * inner * 4);
   f.wqT = (float*)ws.take((size_t)dim * inner * 4);
   f.a32 = (float*)ws.take((size_t)heads * Lp * dim * 4);
   f.b32 = (float*)ws.take((size_t)dim * heads * Lp * 4);
@@ -243,7 +247,10 @@ extern "C" int nrb_latent_fold(int precision, int dim, int heads, int dim_head, 
   NRB_REQUIRE(precision == NRB_F32 || precision == NRB_BF16, "nrb_latent_fold: bad precision");
   NRB_REQUIRE(dim > 0 && dim % 16 == 0, "nrb_latent_fold: dim must be a multiple of 16");
   NRB_REQUIRE(heads > 0 && dim_head > 0 && dim_head % 16 == 0, "nrb_latent_fold: dim_head must be a multiple of 16");
-  NRB_REQUIRE(num_latents > 0 && num_latents % 4 == 0, "nrb_latent_fold: num_latents must be a multiple of 4");
+  NRB_REQUIRE(num_latents > 0, "nrb_latent_fold: num_latents must be positive");
+  NRB_REQUIRE(precision != NRB_BF16 || heads * pad_latents(num_latents) % 64 == 0,
+              "nrb_latent_fold: bf16 needs heads * latents_padded to be a multiple of 64 (got %d x %d)", heads,
+              pad_latents(num_latents));
   NRB_REQUIRE(latents && ln_ctx_w && ln_ctx_b && w_q && w_kv && w_out && a_out && b_out && workspace,
               "nrb_latent_fold: null pointer");
   FoldWs f = fold_ws(workspace, dim, heads, dim_head, num_latents);
@@ -252,29 +259,30 @@ extern "C" int nrb_latent_fold(int precision, int dim, int heads, int dim_head, 
     return NRB_E_WORKSPACE;
   }
   cudaStream_t st = as_stream(stream);
-  const int L = num_latents, Lp = pad_latents(L), inner = heads * dim_head, hl = heads * Lp;
+  const int L = num_latents, L4 = fold_latents(L), Lp = pad_latents(L), inner = heads * dim_head, hl = heads * Lp;
   int rc;
   // context = LN_ctx(latents); kv = to_kv(context)            (latent_attention.py:18-19, 67)
+  if (L4 > L) NRB_CUDA_CHECK(cudaMemsetAsync(f.cn + (size_t)L * dim, 0, (size_t)(L4 - L) * dim * 4, st));
   if ((rc = layer_norm_rows(latents, NRB_F32, dim, nullptr, ln_ctx_w, ln_ctx_b, f.cn, NRB_F32, dim, nullptr, 0, L,
                             nullptr, dim, st)) != NRB_OK)
     return rc;
-  if ((rc = gemm_f32_simt(NRB_EPI_NONE, NRB_F32, f.cn, dim, w_kv, dim, nullptr, nullptr, 0, f.kv, 2 * inner, L,
+  if ((rc = gemm_f32_simt(NRB_EPI_NONE, NRB_F32, f.cn, dim, w_kv, dim, nullptr, nullptr, 0, f.kv, 2 * inner, L4,
                           nullptr, 2 * inner, dim, st)) != NRB_OK)
     return rc;
   // fold the SDPA scale dim_head^-0.5 (:69-72) into K
-  if ((rc = scale_cols_f32(f.kv, 2 * inner, L, inner, 1.0f / sqrtf((float)dim_head), st)) != NRB_OK) return rc;
+  if ((rc = scale_cols_f32(f.kv, 2 * inner, L4, inner, 1.0f / sqrtf((float)dim_head), st)) != NRB_OK) return rc;
   if ((rc = transpose_f32(w_q, inner, dim, f.wqT, st)) != NRB_OK) return rc;
   NRB_CUDA_CHECK(cudaMemsetAsync(f.a32, 0, (size_t)hl * dim * 4, st));
   NRB_CUDA_CHECK(cudaMemsetAsync(f.b32, 0, (size_t)dim * hl * 4, st));
   for (int h = 0; h < heads; ++h) {
     // A_h[l, i] = sum_c K[l, h*dh+c] * Wq[h*dh+c, i]
     if ((rc = gemm_f32_simt(NRB_EPI_NONE, NRB_F32, f.kv + h * dim_head, 2 * inner, f.wqT + h * dim_head, inner,
-                            nullptr, nullptr, 0, f.a32 + (size_t)h * Lp * dim, dim, L, nullptr, dim, dim_head,
+                            nullptr, nullptr, 0, f.a32 + (size_t)h * Lp * dim, dim, L4, nullptr, dim, dim_head,
                             st)) != NRB_OK)
       return rc;
     // B[i, h*Lp + l] = sum_c Wout[i, h*dh+c] * V[l, h*dh+c]
     if ((rc = gemm_f32_simt(NRB_EPI_NONE, NRB_F32, w_out + h * dim_head, inner, f.kv + inner + h * dim_head,
-                            2 * inner, nullptr, nullptr, 0, f.b32 + (size_t)h * Lp, hl, dim, nullptr, L, dim_head,
+                            2 * inner, nullptr, nullptr, 0, f.b32 + (size_t)h * Lp, hl, dim, nullptr, L4, dim_head,
                             st)) != NRB_OK)
       return rc;
   }

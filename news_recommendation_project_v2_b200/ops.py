@@ -366,11 +366,15 @@ class FoldedLatent:
 
 def latent_fold(sd: dict, heads: int, dim_head: int, precision: torch.dtype, device) -> FoldedLatent:
     """One-time weight preparation (nrb_latent_fold + GEGLU row interleave)."""
+    L, dim = sd["latents"].shape
+    Lp = max(32, 1 << (L - 1).bit_length())  # power of two: softmax groups tile the 256-column MMA tiles
+    if precision == torch.bfloat16 and heads * Lp % 64:
+        # the value GEMM contracts over heads * Lp, and the tensor-core GEMM takes K in multiples of 64
+        raise _lib.NrbError(f"bf16 latent attention needs heads * latents_padded to be a multiple of 64 "
+                            f"(got {heads} x {Lp}); use an even head count, more than 32 latents or fp32")
     dev = require_device(device)
     f32 = lambda k: sd[k].detach().to(device=dev, dtype=torch.float32).contiguous()
     lat = f32("latents")
-    L, dim = lat.shape
-    Lp = max(32, 1 << (L - 1).bit_length())  # power of two: softmax groups tile the 256-column MMA tiles
     p0, p1 = "cross_attend_blocks.0.", "cross_attend_blocks.1."
     wq, wkv, wout = f32(p0 + "fn.to_q.weight"), f32(p0 + "fn.to_kv.weight"), f32(p0 + "fn.to_out.weight")
     if wq.shape != (heads * dim_head, dim):

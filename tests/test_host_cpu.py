@@ -67,6 +67,18 @@ def test_argument_validation_without_gpu():
     assert lib.nrb_push_attach(None, 0, 0) == -1 and b"spread" in lib.nrb_last_error()
     lib.nrb_push_cancel()
     assert lib.nrb_push_flush(None) == 0  # nothing pending: no launch, no CUDA call
+    # latent fold: any latent count passes the size checks (here it stops at the null pointers); bf16 with
+    # heads * latents_padded not a multiple of 64 is refused by name, in the library and before any device work in ops
+    assert lib.nrb_latent_fold(0, 64, 2, 32, 50, *[None] * 9, 0, None) == -1 and b"null" in lib.nrb_last_error()
+    assert lib.nrb_latent_fold(1, 64, 1, 32, 409, *[None] * 9, 0, None) == -1 and b"null" in lib.nrb_last_error()
+    assert lib.nrb_latent_fold(1, 64, 1, 32, 32, *[None] * 9, 0, None) == -1
+    assert b"heads * latents_padded" in lib.nrb_last_error() and b"1 x 32" in lib.nrb_last_error()
+    # (the fold's FFMA GEMMs run over the latent count rounded up to a multiple of 4)
+    assert lib.nrb_latent_fold_workspace_bytes(64, 2, 32, 50) == lib.nrb_latent_fold_workspace_bytes(64, 2, 32, 52)
+    from news_recommendation_project_v2_b200 import ops, synthetic as syn
+    sd = syn.make_latent_state_dict(64, 20, heads=3, dim_head=32, seed=0)
+    with pytest.raises(_lib.NrbError, match=r"heads \* latents_padded .*\(got 3 x 32\)"):
+        ops.latent_fold(sd, 3, 32, torch.bfloat16, None)
 
 
 def test_host_copy_is_exact_for_any_thread_count():
