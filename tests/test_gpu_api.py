@@ -338,12 +338,67 @@ def test_mind_metrics_kernel_matches_reference_golden(golden_dir):
         y = labels_l[i].astype(np.float32)
         ys = 1.0 / ranks_l[i]
         order = np.argsort(ys, kind="stable")[::-1]
+        ideal = np.argsort(y, kind="stable")[::-1]
         want_mrr = np.sum(np.take(y, order) / (np.arange(len(y)) + 1)) / y.sum()
         auc = oracle._auc_tie_aware(y, ys)
         assert abs(per[i, 0] - auc) < 1e-12 and abs(per[i, 1] - want_mrr) < 1e-12
+        dcg = lambda o, k: np.sum((2.0 ** y[o[:k]] - 1) / np.log2(np.arange(len(o[:k])) + 2))
+        assert abs(per[i, 2] - dcg(order, 5) / dcg(ideal, 5)) < 1e-12
+        assert abs(per[i, 3] - dcg(order, 10) / dcg(ideal, 10)) < 1e-12
     assert np.isnan(per[3]).all() and int(sums[4].item()) == 3
     with pytest.raises(ValueError):
         score(ranks_l, labels_l)
+
+
+def test_mind_metrics_kernel_several_impressions_per_warp():
+    """nrb_mind_metrics with every warp of its grid (SMs x 16 CTAs x 8 warps) on >= 3 impressions, against the
+    vectorised fp64 score_row (stable tie order): the `large` candidate counts plus 600 / 1,500 (global-memory path),
+    heavy rank ties, label-2 gains, single-class, NaN-group and empty impressions next to ordinary ones on one warp."""
+    from news_recommendation_project_v2_b200 import ops
+    from tests import segment_oracle as so
+    W = torch.cuda.get_device_properties(0).multi_processor_count * 16 * 8
+    n_imp = 3 * W + W // 6
+    assert n_imp // W >= 3 and n_imp >= 3 * W
+    rng = np.random.default_rng(12)
+    counts = np.clip(np.rint(rng.lognormal(np.log(30.0), 0.7, size=n_imp)), 2, 300).astype(np.int64)
+    counts[[3, W + 7, 2 * W + 11]] = 600
+    counts[[5, W + 9, 3 * W + 1]] = 1500
+    empty, zero_rank, all_neg, all_pos = [W + 13, 2], [17, 2 * W + 17], [19, 2 * W + 3], [W + 21, 23]
+    counts[empty] = 0
+    off = so.csr(counts)
+    n = int(off[-1])
+    scores = rng.integers(0, 8, size=n).astype(np.float32)  # heavy ties: at most 8 distinct scores per impression
+    scores[off[3]:off[4]] = rng.integers(0, 200, size=600)
+    ranks, _ = so.dense_rank_segments(torch.from_numpy(scores), torch.from_numpy(off))
+    ranks = ranks.numpy()
+    labels = (rng.random(n) < 0.3).astype(np.int8)
+    starts = off[:-1][counts > 0]
+    labels[starts], labels[starts + 1] = 1, 0  # both classes
+    two = rng.choice(n_imp, size=n_imp // 50, replace=False)
+    two = np.union1d(two[counts[two] > 0], [0, W, 2 * W, 3])
+    labels[off[two]] = 2  # gains 2^y - 1 = 3
+    for i in zero_rank:
+        ranks[off[i]:off[i + 1]] = 0  # a NaN group's sentinel
+    for i, v in [(i, 0) for i in all_neg] + [(i, 1) for i in all_pos]:
+        labels[off[i]:off[i + 1]] = v
+    want = so.mind_metrics_segments(ranks, labels, counts)
+    invalid = np.isnan(want[:, 0])
+    assert np.array_equal(np.flatnonzero(invalid), np.sort(empty + zero_rank + all_neg + all_pos))
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).cuda()
+    per, sums = ops.mind_metrics(t(ranks), t(labels), t(off))
+    per, sums = per.cpu().numpy(), sums.cpu().numpy()
+    assert np.array_equal(np.isnan(per), np.isnan(want))
+    np.testing.assert_allclose(per, want, atol=1e-12, rtol=0)
+    print(f"\nmind metrics: {n_imp} impressions on {W} warps, max |err| {np.abs(per - want)[~invalid].max():.2e}")
+    want_sums = want[~invalid].sum(0)
+    # atomics in a varying order: 1e-9 relative
+    np.testing.assert_allclose(sums[:4], want_sums, rtol=1e-9, atol=0)
+    assert sums[4] == (~invalid).sum()
+    none, sums2 = ops.mind_metrics(t(ranks), t(labels), t(off), want_per_impression=False)
+    sums2 = sums2.cpu().numpy()
+    assert none is None
+    np.testing.assert_allclose(sums2[:4], want_sums, rtol=1e-9, atol=0)
+    assert sums2[4] == (~invalid).sum()
 
 
 @pytest.mark.parametrize("precision,tol", [("fp32", 2e-5), ("bf16", 3e-2)])

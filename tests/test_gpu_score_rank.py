@@ -11,6 +11,7 @@ import torch
 
 from oracle import oracle
 from news_recommendation_project_v2_b200 import synthetic as syn
+from tests import segment_oracle as so
 
 pytestmark = pytest.mark.gpu
 
@@ -23,6 +24,10 @@ def ops():
 
 def _csr(lengths):
     return torch.from_numpy(syn.csr_offsets(np.asarray(lengths))).cuda()
+
+
+def _sms():
+    return torch.cuda.get_device_properties(0).multi_processor_count
 
 
 def test_dense_rank_bit_exact(ops, golden_dir):
@@ -42,6 +47,24 @@ def test_dense_rank_bit_exact(ops, golden_dir):
     got = ops.dense_rank(torch.from_numpy(scores).cuda(), _csr(counts)).cpu().numpy()
     want = np.concatenate([np.asarray(r) for r in oracle.rank_group_preds(scores, counts)])
     assert np.array_equal(got, want.astype(np.int32))
+    # every warp on >= 3 groups: fp32 scores run on SMs x 32 CTAs of 8 warps, float64 on SMs x 32 CTAs of 4 warps;
+    # the reference ranks all groups at once (tests/segment_oracle.py, held to rank_group_preds on the CPU)
+    W = _sms() * 32 * 8
+    n_groups = 3 * W + 1001
+    assert n_groups // W >= 3 and n_groups // (_sms() * 32 * 4) >= 3
+    counts = rng.integers(0, 70, size=n_groups).astype(np.int64)
+    counts[[5, W + 5, 2 * W + 6, 3 * W + 7]] = [700, 0, 513, 1000]  # global-memory path / empty, next to small groups
+    off = syn.csr_offsets(counts)
+    n = int(off[-1])
+    for dt in (np.float32, np.float64):
+        scores = (rng.integers(-8, 9, size=n) / 4.0).astype(dt)  # heavy ties
+        scores[n // 2:] = rng.standard_normal(n - n // 2)
+        if dt == np.float64:  # differences below fp32 resolution stay distinct
+            scores[: n // 2] += rng.integers(0, 2, size=n // 2) * 2.0 ** -40
+        scores[[off[W + 9] + 1, off[2 * W + 6] + 100]] = np.nan  # NaN groups rank 0 (one on the global path)
+        sc = torch.from_numpy(scores).cuda()
+        want, _ = so.dense_rank_segments(sc, torch.from_numpy(off).cuda())
+        assert torch.equal(ops.dense_rank(sc, torch.from_numpy(off).cuda()), want)
 
 
 def test_gather_collate_bit_exact(ops, golden_dir):
@@ -62,6 +85,22 @@ def test_gather_collate_bit_exact(ops, golden_dir):
         emb, mask = ops.gather_collate(table.cuda(), torch.from_numpy(imp.hist_idx).cuda(), _csr(imp.hist_len),
                                        int(imp.hist_len.max()))
         assert torch.equal(emb.cpu(), want_e.to(dt)) and torch.equal(mask.cpu(), want_m)
+    # every warp of the grid (SMs x 32 CTAs of 8 warps, one warp per (group, slot)) on >= 4 slots
+    W = _sms() * 32 * 8
+    max_len = 64
+    n_groups = -(-4 * W // max_len) + 3
+    assert n_groups * max_len >= 4 * W
+    rng = np.random.default_rng(4)
+    lens = rng.integers(0, max_len + 1, size=n_groups).astype(np.int64)
+    lens[[1, n_groups // 2]] = [max_len, 0]
+    idx = torch.from_numpy(rng.integers(0, 5000, size=int(lens.sum())).astype(np.int32)).cuda()
+    valid = torch.arange(max_len, device="cuda")[None, :] < torch.from_numpy(lens).cuda()[:, None]
+    for dt in (torch.float32, torch.bfloat16):
+        big = syn.make_table(5000, 256, seed=8).to(dt).cuda()
+        emb, mask = ops.gather_collate(big, idx, _csr(lens), max_len)
+        want = torch.zeros(n_groups, max_len, 256, dtype=dt, device="cuda")
+        want[valid] = big[idx.long()]
+        assert torch.equal(emb, want) and torch.equal(mask, valid.to(torch.int32))
     with pytest.raises(IndexError):
         ops.gather_collate(table.cuda(), torch.tensor([1, 500], dtype=torch.int32).cuda(), _csr([2]), 2)
 
@@ -209,6 +248,20 @@ def test_topk_order_bit_exact(ops):
             want = np.full(k, -1, dtype=np.int32)
             want[:min(k, len(s))] = order[:k]
             assert np.array_equal(got[g], want), (g, k)
+    # every warp of the grid (SMs x 32 CTAs of 8 warps) on >= 3 groups, most of them shorter than k = 37; the
+    # reference orders all groups at once (tests/segment_oracle.py, held to the loop above on the CPU)
+    W = _sms() * 32 * 8
+    n_groups = 3 * W + 777
+    assert n_groups // W >= 3
+    counts = rng.integers(0, 60, size=n_groups).astype(np.int32)
+    counts[[3, W + 3, 2 * W + 3]] = [700, 0, 2]
+    off = syn.csr_offsets(counts)
+    scores = (rng.integers(-6, 7, size=int(off[-1])) / 4.0).astype(np.float32)
+    scores[[off[W + 4], off[2 * W + 5] + 1, off[3] + 600]] = np.nan
+    ks = (1, 5, 10, 37)
+    for k, want in zip(ks, so.topk_order_segments(scores, counts, ks)):
+        got = ops.topk_order(torch.from_numpy(scores).cuda(), _csr(counts), k).cpu().numpy()
+        assert np.array_equal(got, want), k
 
 
 def test_rank_group_preds_float64_not_merged_below_fp32(ops):
@@ -270,3 +323,20 @@ def test_score_host_int16_ranks_equal_int32(ops):
     assert int(out[100]) == 101 and int(out[-1]) == 32767
     with pytest.raises(OverflowError):
         ops.raise_on_index_error(flag, "narrow")
+    # past one pass of the grid-stride loop (SMs x 16 CTAs x 256 threads x 8 ranks), with a scalar tail (n % 8 = 3)
+    n = 5_000_003
+    assert n // 8 > _sms() * 16 * 256 and n % 8 != 0
+    g = torch.Generator(device="cuda").manual_seed(6)
+    ranks = torch.randint(1, 32768, (n,), dtype=torch.int32, device="cuda", generator=g)
+    flag = ops.new_err_flag(torch.device("cuda"))
+    out = ops.narrow_ranks(ranks, torch.empty(n, dtype=torch.int16, device="cuda"), flag)
+    assert torch.equal(out.to(torch.int32), ranks) and int(flag.item()) == 0
+    for at in (n - 11, n - 2):  # the second pass of the 8-wide loop, the scalar tail
+        r = ranks.clone()
+        r[at] = 40000
+        flag = ops.new_err_flag(torch.device("cuda"))
+        out = ops.narrow_ranks(r, torch.full((n,), -5, dtype=torch.int16, device="cuda"), flag)
+        want = r.clamp_max(32767)
+        assert torch.equal(out.to(torch.int32), want) and int(out[at]) == 32767
+        with pytest.raises(OverflowError):
+            ops.raise_on_index_error(flag, "narrow")

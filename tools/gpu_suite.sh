@@ -4,8 +4,9 @@
 mkdir -p gpurun_out
 nvidia-smi --query-gpu=name,driver_version,memory.total,clocks.max.sm --format=csv > gpurun_out/gpu_info.txt 2>&1
 status=0
-for f in test_gpu_score_rank test_gpu_dense test_gpu_latent test_gpu_api test_gpu_fullsize test_gpu_multi; do
-  timeout -k 10 900 python -m pytest tests/$f.py -q -m gpu --maxfail=12 --no-header -p no:cacheprovider ${1:+-k "$1"} \
+for path in tests/test_gpu_*.py; do
+  f=$(basename "$path" .py)
+  timeout -k 10 900 python -m pytest "$path" -q -m gpu --maxfail=12 --no-header -p no:cacheprovider ${1:+-k "$1"} \
       > gpurun_out/$f.log 2>&1
   rc=$?
   echo "== $f exit $rc"
