@@ -52,6 +52,7 @@ extern "C" {
 #define NRB_EPI_GEGLU 4     /* y[j] = a_j * gelu_erf(g_j), W rows interleaved in pairs (a0,a1,g0,g1,a2,a3,g2,g3..) latent_attention.py:24-27 */
 #define NRB_EPI_SOFTMAX 5   /* y = softmax over each group of `group` columns (first `group_valid` valid); latent_attention.py:69-72 */
 #define NRB_EPI_TOPK 6      /* internal to nrb_recommend: per-row top-k of acc * scale[col], no output tile */
+#define NRB_EPI_TOPK_BLEND 7 /* internal to nrb_recommend_pool_blend: the same of acc * scale[col] blended with base[col] */
 
 typedef void* nrb_stream_t;
 
@@ -261,6 +262,34 @@ int nrb_recommend(int precision, int dim, int64_t n_rows, const void* table, int
                   const int32_t* excl_idx, const int64_t* excl_off, int64_t n_excl, int k,
                   int32_t* out_rows, float* out_scores, int32_t* err_flag, void* workspace, size_t workspace_bytes,
                   nrb_stream_t stream);
+
+/* nrb_recommend from a pool of the table's rows, with the classification-baseline blend of nrb_score_rank.
+ * (nrb_recommend is this call with n_pool = -1 and cand_base = NULL.)  Arguments of nrb_recommend, plus:
+ *   pool / n_pool   : int32 table row ids, strictly ascending, in [0, n_rows): only these rows are eligible, and the
+ *                     GEMM runs over them alone (their rows of table_op are gathered into the workspace, so table_op
+ *                     must then be 16-byte aligned with a 16-byte multiple row pitch).  A violation sets bit 0 of
+ *                     *err_flag.  n_pool < 0: the whole table (pool ignored).  n_pool = 0: every list is padding and
+ *                     no GEMM runs.  Returned ids are table row ids; excluded ids outside the pool are ignored but
+ *                     still range-checked against n_rows.
+ *   cand_base       : optional fp32 [n_rows] per-row baseline (NULL: pure cosine), blend_alpha its weight:
+ *                       score = cos * blend_alpha + cand_base[r] * (1 - blend_alpha)   for users with a history,
+ *                       score = cand_base[r]                                           for users without one
+ *                     (the expression and the fallback of nrb_score_rank; the fallback is a select, so the NaN vector
+ *                     a mean-pool encoder gives an empty history never scores).  A row whose baseline is NaN is never
+ *                     returned.
+ *   hist_off        : optional int64 [n_users + 1] history offsets; user u has no history when
+ *                     hist_off[u + 1] == hist_off[u].  NULL: every user has one.  Separate from excl_off so that the
+ *                     fallback holds when the history is not excluded.
+ * Order, padding, limits and the dependence on the other users of the call are those of nrb_recommend, with the
+ * GEMM configuration chosen by n_users alone. */
+size_t nrb_recommend_pool_blend_workspace_bytes(int precision, int dim, int64_t n_rows, int64_t n_users,
+                                                int64_t n_excl, int k, int64_t n_pool);
+int nrb_recommend_pool_blend(int precision, int dim, int64_t n_rows, const void* table, int64_t table_stride,
+                             const void* table_op, int64_t op_stride, const float* users, int64_t users_stride,
+                             int64_t n_users, const int32_t* excl_idx, const int64_t* excl_off, int64_t n_excl, int k,
+                             const int32_t* pool, int64_t n_pool, const float* cand_base, float blend_alpha,
+                             const int64_t* hist_off, int32_t* out_rows, float* out_scores, int32_t* err_flag,
+                             void* workspace, size_t workspace_bytes, nrb_stream_t stream);
 
 /* ---- MIND metrics on device (consumer of the ranks; "next" row of the hot path) ---------------
  * replaces evaluation.py:34-98 (score_row per impression in a 4-process pool + mean):

@@ -98,6 +98,10 @@ PROTOTYPES = {
     "nrb_recommend": (_i32, [_i32, _i32, _i64, _c_void_p, _i64, _c_void_p, _i64, _c_void_p, _i64, _i64,
                              _c_void_p, _c_void_p, _i64, _i32, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _sz,
                              _c_void_p]),
+    "nrb_recommend_pool_blend_workspace_bytes": (_sz, [_i32, _i32, _i64, _i64, _i64, _i32, _i64]),
+    "nrb_recommend_pool_blend": (_i32, [_i32, _i32, _i64, _c_void_p, _i64, _c_void_p, _i64, _c_void_p, _i64, _i64,
+                                        _c_void_p, _c_void_p, _i64, _i32, _c_void_p, _i64, _c_void_p, _f32,
+                                        _c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _sz, _c_void_p]),
 }
 
 _lock = threading.Lock()

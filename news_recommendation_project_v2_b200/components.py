@@ -4,7 +4,7 @@
   SaveEmbeddingComponent     components.py:178-222  table writer  (`<dataset>.pt`, `query_<dataset>.pt`)
   LoadEmbeddingComponent     components.py:225-258  table reader
   FinalAttentionComponent    components.py:980-1027 gather + user encoder + cosine + dense rank
-  TopKRecommendationComponent (new)                 the k best news of the whole table per user
+  TopKRecommendationComponent (new)                 the k best news of the table (or of the impressions) per user
 
 Only `transform` is in scope (scripts/eval.py's path); training stays with the reference."""
 from __future__ import annotations
@@ -15,7 +15,7 @@ from typing import Any, Optional
 import numpy as np
 import torch
 
-from .data_model_helper import get_final_second_attention_score, get_top_k_recommendations
+from .data_model_helper import get_classification_preds, get_final_second_attention_score, get_top_k_recommendations
 from .data_utils import split_impressions_and_history
 from .modeling_utils import get_final_attention_model
 from .pipeline import PipelineComponent, check_req_keys
@@ -118,25 +118,45 @@ class TopKRecommendationComponent(PipelineComponent):
     """Recommends, for every user with a history, the k news of the whole table that score best against the user
     vector (the cosine FinalAttentionComponent ranks candidates by), history excluded by default.  Adds
     `top_k_rows` (int32 [U, k] row ids), `top_k_scores` (float32 [U, k]) and `top_k_news` (object [U, k] news ids
-    from `news_list`, None where a user has fewer than k eligible news)."""
+    from `news_list`, None where a user has fewer than k eligible news).
+
+    With `classification_model` the news are scored like `get_final_score`: the cosine blended with the model's
+    per-news classification score (weight of `weight_model`), and users without a history get the classification
+    score alone; the context then needs `history_bool` and there is one list per behaviour row.
+    `restrict_to_impressions` draws the news from those that occur in `impression_rev_ind_array` only."""
 
     required_keys = {"news_embeddings", "history_rev_ind_array", "history_len_list", "news_list"}
 
     def __init__(self, k: int = 10, attention_model_path: Optional[Path] = None, attention_model=None,
-                 exclude_history: bool = True, precision=None, **_unused):
+                 exclude_history: bool = True, precision=None, classification_model=None, weight_model=None,
+                 restrict_to_impressions: bool = False, **_unused):
         self.k = int(k)
         self.attention_model = attention_model if attention_model is not None else \
             get_final_attention_model(attention_model_path)
         self.exclude_history = exclude_history
         self.precision = precision
+        self.classification_model = classification_model
+        self.weight_model = weight_model
+        self.restrict_to_impressions = restrict_to_impressions
 
     def transform(self, context_dict: dict[str, Any]) -> dict[str, Any]:
-        check_req_keys(self.required_keys, context_dict)
+        req = set(self.required_keys)
+        if self.classification_model is not None:
+            req.add("history_bool")
+        if self.restrict_to_impressions:
+            req.add("impression_rev_ind_array")
+        check_req_keys(req, context_dict)
         out = context_dict.copy()
+        extra = {}
+        if self.classification_model is not None:
+            extra = {"classification_score": get_classification_preds(out["news_embeddings"], self.classification_model),
+                     "weight_model": self.weight_model, "history_bool": out["history_bool"]}
+        if self.restrict_to_impressions:
+            extra["pool"] = np.unique(np.asarray(out["impression_rev_ind_array"][0]))
         res = get_top_k_recommendations(
             out["history_rev_ind_array"][0], out["history_len_list"], out["news_embeddings"], self.attention_model,
             k=self.k, exclude_history=self.exclude_history, query_news_embeddings=out.get("query_news_embeddings"),
-            precision=self.precision)
+            precision=self.precision, **extra)
         out.update(res)
         news = np.asarray(out["news_list"], dtype=object)
         rows = res["top_k_rows"]

@@ -10,7 +10,7 @@ int gemm_bf16_tc(int epi, int out_dtype, const void* a, int64_t lda, const void*
                  const void* res, int64_t ldres, void* y, int64_t ldy, int64_t M, const int* m_dev, int N, int K,
                  int group, int group_valid, cudaStream_t st, int res_dtype = NRB_F32,
                  const int32_t* res_map = nullptr);
-// gemm_tc.cu -- tcgen05 GEMM with the fused top-k epilogue (NRB_EPI_TOPK)
+// gemm_tc.cu -- tcgen05 GEMM with the fused top-k epilogue (NRB_EPI_TOPK, or NRB_EPI_TOPK_BLEND when base != NULL)
 struct TopkPlan {
   int cg;              // 1: single CTA (M <= 128), 2: CTA pairs
   int rows_per_block;  // 128 * cg
@@ -23,7 +23,7 @@ __host__ __device__ inline int64_t topk_owner(const TopkPlan& t, int64_t u) {
 TopkPlan topk_plan(int64_t M, int64_t N);
 int gemm_topk_tc(const void* a, int64_t lda, const void* w, int64_t ldw, const float* scale, const int64_t* excl_off,
                  const int32_t* excl_sorted, int64_t M, int N, int K, int k, const TopkPlan& plan, void* parts,
-                 cudaStream_t st);
+                 const float* base, const uint8_t* cold, float alpha, cudaStream_t st);
 // gemm_simt.cu -- FFMA (fp32 operands)
 int gemm_f32_simt(int epi, int out_dtype, const void* a, int64_t lda, const void* w, int64_t ldw,
                   const float* bias, const void* res, int64_t ldres, void* y, int64_t ldy, int64_t M,

@@ -51,7 +51,8 @@ struct GemmCfg {
   static_assert(CG == 1 || (CG == 2 && BN == 256 && EPI != NRB_EPI_SOFTMAX), "CTA pairs: 256-wide tiles, no softmax");
   static constexpr bool kStaged = OUT_BF16;
   static constexpr bool kSoftmax = EPI == NRB_EPI_SOFTMAX;
-  static constexpr bool kTopk = EPI == NRB_EPI_TOPK;
+  static constexpr bool kTopk = EPI == NRB_EPI_TOPK || EPI == NRB_EPI_TOPK_BLEND;
+  static constexpr bool kBlend = EPI == NRB_EPI_TOPK_BLEND;
   // fp32 outputs: every epilogue warp transposes its 32x32 accumulator chunk through a private 4 KB smem patch so
   // that the residual loads and the output stores touch 4 rows x 128 contiguous bytes per instruction instead of
   // 32 rows x 16 bytes (GEGLU with fp32 output -- unused on the hot path -- keeps the direct row-per-lane stores)
@@ -101,6 +102,10 @@ struct GemmParams {
   //   y       = partial lists, 8-byte (score, column) entries [rows][2 halves][ldy slots][group]
   //   ldy     = slots per (row, half): CTAs (pairs) whose contiguous unit range touches one row block
   //   group   = k
+  // NRB_EPI_TOPK_BLEND adds (appended, so that the offsets of every other field stay as they are):
+  const float* topk_base;    // per-column baseline, NaN from column N up to the next multiple of 256
+  const uint8_t* topk_cold;  // per row: 1 = empty history, the score is topk_base alone
+  float topk_alpha;          // score = acc * scale * alpha + base * (1 - alpha) for the other rows
 };
 
 __device__ __forceinline__ float ex2_approx(float x) {
@@ -437,6 +442,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     int topk_cnt = 0;            // top-k: entries in this thread's list
     float topk_thr = -INFINITY;  // top-k: score a column must beat (the k-th best once the list is full)
     int64_t hcur = 0, hend = 0;  // top-k: cursor into this row's sorted excluded columns
+    bool topk_cold = false;      // top-k blend: this row scores by the baseline alone
     // accumulator hand-back: the (leader's) MMA warp waits for every epilogue warp of the pair
     auto release_tmem = [&](int a) {
       // (TMEM reads are ordered by tcgen05.fence::before_thread_sync; no memory release is needed, which
@@ -591,6 +597,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         }
       } else if constexpr (Cfg::kTopk) {
         // ---------- top-k: score = acc * scale[col]; columns that beat the k-th best enter a smem list ----------
+        // (blend: score = cold ? base[col] : acc * scale[col] * alpha + base[col] * (1 - alpha), a select so that a
+        //  NaN user vector of an empty history cannot reach the list)
         const int k = p.group;
         const int64_t m_u = u / n_units_per_row;  // row block of the unit
         uint2* const list = topk_list + (e * 32 + lane);
@@ -600,6 +608,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           topk_cnt = 0;
           topk_thr = -INFINITY;
           hcur = hend = 0;
+          if constexpr (Cfg::kBlend) topk_cold = row_ok && p.topk_cold[row] != 0;
           if (p.res != nullptr && row_ok) {
             const int64_t* ho = reinterpret_cast<const int64_t*>(p.res);
             int64_t lo = ho[row], hi = ho[row + 1];
@@ -655,6 +664,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             v[j + 1] = __uint_as_float(r[j + 1]) * sc.y;
             v[j + 2] = __uint_as_float(r[j + 2]) * sc.z;
             v[j + 3] = __uint_as_float(r[j + 3]) * sc.w;
+            if constexpr (Cfg::kBlend) {  // base is NaN past column N as well: cold rows never score the zero fill
+              const float4 b = *reinterpret_cast<const float4*>(p.topk_base + col0 + j);
+              const float a = p.topk_alpha, oma = 1.0f - p.topk_alpha;
+              v[j] = topk_cold ? b.x : v[j] * a + b.x * oma;
+              v[j + 1] = topk_cold ? b.y : v[j + 1] * a + b.y * oma;
+              v[j + 2] = topk_cold ? b.z : v[j + 2] * a + b.z * oma;
+              v[j + 3] = topk_cold ? b.w : v[j + 3] * a + b.w * oma;
+            }
             any |= (v[j] > topk_thr) | (v[j + 1] > topk_thr) | (v[j + 2] > topk_thr) | (v[j + 3] > topk_thr);
           }
           if (any) {  // rare once the list is full
@@ -1036,10 +1053,11 @@ TopkPlan topk_plan(int64_t M, int64_t N) {
   return t;
 }
 
-// Partial top-k lists of (a[M,K] . w[N,K]^T) * scale[N] per row: see GemmParams for the NRB_EPI_TOPK fields.
+// Partial top-k lists of (a[M,K] . w[N,K]^T) * scale[N] per row, blended with base[N] when base != NULL: see
+// GemmParams for the NRB_EPI_TOPK / NRB_EPI_TOPK_BLEND fields.
 int gemm_topk_tc(const void* a, int64_t lda, const void* w, int64_t ldw, const float* scale, const int64_t* excl_off,
                  const int32_t* excl_sorted, int64_t M, int N, int K, int k, const TopkPlan& plan, void* parts,
-                 cudaStream_t st) {
+                 const float* base, const uint8_t* cold, float alpha, cudaStream_t st) {
   NRB_REQUIRE(M > 0 && N > 0 && K > 0 && K % kBK == 0, "nrb_recommend: bad GEMM shape");
   NRB_REQUIRE(k >= 1 && k <= kTopkMaxK, "nrb_recommend: k must be in [1, %d]", kTopkMaxK);
   CUtensorMap ma, mw;
@@ -1061,6 +1079,13 @@ int gemm_topk_tc(const void* a, int64_t lda, const void* w, int64_t ldw, const f
   p.group = k;
   p.cluster = 1;
   p.push.n_seg = 0;  // the all-gather rides on the dense row kernels only
+  if (base != nullptr) {
+    p.topk_base = base;
+    p.topk_cold = cold;
+    p.topk_alpha = alpha;
+    if (plan.cg == 2) return launch_gemm<256, NRB_EPI_TOPK_BLEND, false, 2>(ma, mw, ma, p, st);
+    return launch_gemm<256, NRB_EPI_TOPK_BLEND, false, 1>(ma, mw, ma, p, st);
+  }
   if (plan.cg == 2) return launch_gemm<256, NRB_EPI_TOPK, false, 2>(ma, mw, ma, p, st);
   return launch_gemm<256, NRB_EPI_TOPK, false, 1>(ma, mw, ma, p, st);
 }

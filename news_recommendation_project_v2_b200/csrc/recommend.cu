@@ -1,13 +1,19 @@
-// Whole-table retrieval: the k best rows of the resident table for each user (nrb_recommend).
+// Retrieval: the k best rows of the resident table, or of a pool of its rows, for each user (nrb_recommend,
+// nrb_recommend_pool_blend).
 //
-//   score(u, r) = (u / max(|u|, 1e-8)) . c_r / max(|c_r|, 1e-8)      -- the cosine nrb_score_rank computes
+//   cos(u, r)   = (u / max(|u|, 1e-8)) . c_r / max(|c_r|, 1e-8)      -- the cosine nrb_score_rank computes
+//   score(u, r) = cos(u, r); with a baseline: cos * alpha + base[r] * (1 - alpha), or base[r] alone for a user with
+//                 an empty history (a select: a NaN user vector cannot reach the list)
 //
-// One tcgen05 GEMM of the normalised users against the table with a top-k epilogue (gemm_tc.cu, NRB_EPI_TOPK): the
-// scores never leave TMEM.  Around it:
-//   user_operand_kernel  u / max(|u|, 1e-8) -> bf16, or -> [hi|hi|lo] split-bf16 (fp32 tables, K' = 3d)
-//   row_scale_kernel     1 / max(|c_r|, 1e-8) of the stored table (NaN past the last row: never scores)
-//   sort_excl_kernel     each user's excluded rows sorted ascending (any length), range-checked
-//   merge_kernel         one warp per user merges its partial lists into the final [U, k]
+// One tcgen05 GEMM of the normalised users against the table (or the pool's rows of it) with a top-k epilogue
+// (gemm_tc.cu, NRB_EPI_TOPK, or NRB_EPI_TOPK_BLEND with a baseline): the scores never leave TMEM.  Around it:
+//   pool_gather_kernel   the pool's rows of the GEMM operand -> workspace [n_pool, K'], ids validated (pool only)
+//   user_operand_kernel  u / max(|u|, 1e-8) -> bf16, or -> [hi|hi|lo] split-bf16 (fp32 tables, K' = 3d); the
+//                        empty-history flags of the users (baseline only)
+//   row_scale_kernel     1 / max(|c_r|, 1e-8) of the stored table and base[r], in column order (pool order with a
+//                        pool), NaN past the last column: never scores
+//   sort_excl_kernel     each user's excluded rows as columns, sorted ascending (any length), range-checked
+//   merge_kernel         one warp per user merges its partial lists into the final [U, k], columns -> table rows
 // Order: score descending, equal scores by ascending row id; NaN never returned; (-1, NaN) once rows run out.
 #include "dense.cuh"
 
@@ -18,9 +24,28 @@ namespace nrb {
 constexpr int kRecMaxK = 32;
 constexpr int kSortChunk = 2048;  // excluded ids sorted per shared-memory pass
 
+// One warp per pool entry: copies table_op row pool[i] (16-byte vectors) and checks that the ids are strictly
+// ascending and in [0, n_rows); a bad id sets bit 0 of *err_flag and its row is zero-filled.
+__global__ void __launch_bounds__(256)
+pool_gather_kernel(const __nv_bfloat16* op, int64_t ld, int kdim, const int32_t* pool, int64_t n_pool, int64_t n_rows,
+                   __nv_bfloat16* out, int32_t* err_flag) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp_id = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  const int nv = kdim / 8;
+  for (int64_t i = warp_id; i < n_pool; i += n_warps) {
+    const int32_t id = pool[i];
+    const bool ok = id >= 0 && (int64_t)id < n_rows && (i == 0 || pool[i - 1] < id);
+    if (!ok && lane == 0) atomicOr(err_flag, 1);
+    const uint4* src = reinterpret_cast<const uint4*>(op + (int64_t)(ok ? id : 0) * ld);
+    uint4* dst = reinterpret_cast<uint4*>(out + i * kdim);
+    for (int j = lane; j < nv; j += 32) dst[j] = ok ? src[j] : make_uint4(0u, 0u, 0u, 0u);
+  }
+}
+
 __global__ void __launch_bounds__(256)
 user_operand_kernel(const float* users, int64_t ldu, int64_t n_users, int dim, int split, __nv_bfloat16* out,
-                    int64_t ldo) {
+                    int64_t ldo, const int64_t* hist_off, uint8_t* cold) {
   const int lane = threadIdx.x & 31;
   const int64_t warp_id = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -39,17 +64,23 @@ user_operand_kernel(const float* users, int64_t ldu, int64_t n_users, int dim, i
         o[2 * dim + i] = __float2bfloat16_rn(v - __bfloat162float(hi));
       }
     }
+    if (cold != nullptr && lane == 0) cold[r] = hist_off != nullptr && hist_off[r + 1] <= hist_off[r];
   }
 }
 
+// Column c of the GEMM is table row pool[c] (pool != NULL) or row c; an id outside [0, n_rows) (pool_gather_kernel
+// flags it) gets NaN and never scores.  base_out (when base != NULL): base of the column's row, NaN past the last one.
 __global__ void __launch_bounds__(256)
-row_scale_kernel(const void* table, int dtype, int64_t ld, int64_t n_rows, int dim, int64_t n_pad, float* scale) {
+row_scale_kernel(const void* table, int dtype, int64_t ld, int64_t n_rows, int dim, const int32_t* pool,
+                 int64_t n_cols, int64_t n_pad, float* scale, const float* base, float* base_out) {
   const int lane = threadIdx.x & 31;
   const int64_t warp_id = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-  for (int64_t r = warp_id; r < n_pad; r += n_warps) {
+  for (int64_t c = warp_id; c < n_pad; c += n_warps) {
     float ss = 0.f;
-    if (r < n_rows) {
+    const int64_t r = c >= n_cols ? -1 : pool != nullptr ? (int64_t)pool[c] : c;
+    const bool ok = r >= 0 && r < n_rows;
+    if (ok) {
       if (dtype == NRB_F32) {
         const float* c = reinterpret_cast<const float*>(table) + r * ld;
         for (int i = lane; i < dim; i += 32) ss = fmaf(c[i], c[i], ss);
@@ -62,7 +93,10 @@ row_scale_kernel(const void* table, int dtype, int64_t ld, int64_t n_rows, int d
       }
     }
     ss = warp_sum(ss);
-    if (lane == 0) scale[r] = r < n_rows ? 1.0f / fmaxf(sqrtf(ss), 1e-8f) : __int_as_float(0x7fc00000);
+    if (lane == 0) {
+      scale[c] = ok ? 1.0f / fmaxf(sqrtf(ss), 1e-8f) : __int_as_float(0x7fc00000);
+      if (base != nullptr) base_out[c] = ok ? base[r] : __int_as_float(0x7fc00000);
+    }
   }
 }
 
@@ -86,12 +120,24 @@ __device__ void block_bitonic_sort(int32_t* s, int n_pow2) {
   __syncthreads();
 }
 
+// Column of table row `id` in the ascending pool: its position, or n_pool when the row is not in the pool (the
+// epilogue's cursor never reaches a column >= n_pool, so such an id excludes nothing).
+__device__ __forceinline__ int32_t pool_column(const int32_t* pool, int64_t n_pool, int32_t id) {
+  int64_t lo = 0, hi = n_pool;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (pool[mid] < id) lo = mid + 1; else hi = mid;
+  }
+  return (int32_t)(lo < n_pool && pool[lo] == id ? lo : n_pool);
+}
+
 // One block per user.  Histories up to kSortChunk ids are sorted in shared memory; longer ones are sorted in chunks
 // into `tmp`, then every id goes straight to its final place: its position in its own chunk plus, in every other
-// chunk, the number of ids that precede it (ids of earlier chunks first among equals).
+// chunk, the number of ids that precede it (ids of earlier chunks first among equals).  With a pool the ids are
+// range-checked as table rows, then sorted as GEMM columns (pool_column).
 __global__ void __launch_bounds__(256)
-sort_excl_kernel(const int32_t* idx, const int64_t* off, int64_t n_rows, int32_t* tmp, int32_t* out,
-                 int32_t* err_flag) {
+sort_excl_kernel(const int32_t* idx, const int64_t* off, int64_t n_rows, const int32_t* pool, int64_t n_pool,
+                 int32_t* tmp, int32_t* out, int32_t* err_flag) {
   __shared__ int32_t s[kSortChunk];
   const int64_t g = blockIdx.x;
   const int64_t o0 = off[g], n = off[g + 1] - o0;
@@ -107,6 +153,7 @@ sort_excl_kernel(const int32_t* idx, const int64_t* off, int64_t n_rows, int32_t
       if (i < m) {
         v = idx[o0 + c0 + i];
         bad |= v < 0 || (int64_t)v >= n_rows;
+        if (pool != nullptr) v = pool_column(pool, n_pool, v);
       }
       s[i] = v;
     }
@@ -147,8 +194,10 @@ __device__ __forceinline__ unsigned long long topk_key(uint2 e) {
 
 // One warp per user: k rounds of "best head among the user's sorted partial lists".  Lane l owns lists l, l+32, ...
 // (their heads in shared memory) and keeps the best of them; the winning lane advances its head and rescans.
+// Entries hold GEMM columns; with a pool, column c is table row pool[c] (ascending, so the column order is the row order).
 __global__ void __launch_bounds__(256)
-merge_kernel(const uint2* parts, TopkPlan plan, int64_t n_users, int k, int32_t* out_rows, float* out_scores) {
+merge_kernel(const uint2* parts, TopkPlan plan, int64_t n_users, int k, const int32_t* pool, int32_t* out_rows,
+             float* out_scores) {
   extern __shared__ int32_t heads_all[];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int64_t u = (int64_t)blockIdx.x * (blockDim.x >> 5) + w;
@@ -185,7 +234,8 @@ merge_kernel(const uint2* parts, TopkPlan plan, int64_t n_users, int k, int32_t*
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(kFullMask, m, o));
     if (lane == 0) {
-      out_rows[u * k + j] = m == 0ull ? -1 : (int32_t)(~(uint32_t)m);
+      const int32_t col = (int32_t)(~(uint32_t)m);
+      out_rows[u * k + j] = m == 0ull ? -1 : pool != nullptr ? pool[col] : col;
       const uint32_t ord = (uint32_t)(m >> 32);
       const uint32_t b = (ord & 0x80000000u) ? (ord & 0x7fffffffu) : ~ord;
       out_scores[u * k + j] = m == 0ull ? __int_as_float(0x7fc00000) : __uint_as_float(b);
@@ -201,20 +251,27 @@ merge_kernel(const uint2* parts, TopkPlan plan, int64_t n_users, int k, int32_t*
 
 struct RecLayout {
   void* user_op;
+  void* pool_op;  // the pool's rows of table_op (pool only)
   float* scale;
+  float* base;    // base in column order (baseline only)
+  uint8_t* cold;  // per user: empty history (baseline only)
   int32_t* excl_sorted;
   int32_t* excl_tmp;
   uint2* parts;
   size_t bytes;
 };
 
-static RecLayout rec_layout(void* base, int precision, int dim, int64_t n_rows, int64_t n_users, int64_t n_excl,
-                            int k, const TopkPlan& plan) {
+// n_pool < 0: the whole table.  The plan is the GEMM's over max(columns, 1): an empty pool launches no GEMM.
+static RecLayout rec_layout(void* base, int precision, int dim, int64_t n_users, int64_t n_excl, int k, int64_t n_pool,
+                            const TopkPlan& plan) {
   Workspace ws(base, (size_t)-1);
   RecLayout L;
   const int kdim = precision == NRB_BF16 ? dim : 3 * dim;
   L.user_op = ws.take((size_t)n_users * kdim * 2);
+  L.pool_op = n_pool > 0 ? ws.take((size_t)n_pool * kdim * 2) : nullptr;
   L.scale = (float*)ws.take((size_t)plan.n_per_row * 256 * 4);
+  L.base = (float*)ws.take((size_t)plan.n_per_row * 256 * 4);
+  L.cold = (uint8_t*)ws.take((size_t)n_users);
   L.excl_sorted = (int32_t*)ws.take((size_t)std::max<int64_t>(n_excl, 1) * 4);
   L.excl_tmp = (int32_t*)ws.take((size_t)std::max<int64_t>(n_excl, 1) * 4);
   L.parts = (uint2*)ws.take((size_t)plan.m_tiles * plan.rows_per_block * 2 * plan.slots * k * 8);
@@ -222,7 +279,8 @@ static RecLayout rec_layout(void* base, int precision, int dim, int64_t n_rows, 
   return L;
 }
 
-static int check_recommend_args(int precision, int dim, int64_t n_rows, int64_t n_users, int64_t n_excl, int k) {
+static int check_recommend_args(int precision, int dim, int64_t n_rows, int64_t n_users, int64_t n_excl, int k,
+                                int64_t n_pool) {
   NRB_REQUIRE(precision == NRB_BF16 || precision == NRB_F32, "nrb_recommend: precision must be NRB_BF16 or NRB_F32");
   NRB_REQUIRE(k >= 1 && k <= kRecMaxK,
               "nrb_recommend: k must be in [1, %d] (got %d): each epilogue thread keeps its list in %d shared-memory "
@@ -232,34 +290,51 @@ static int check_recommend_args(int precision, int dim, int64_t n_rows, int64_t 
   NRB_REQUIRE(n_rows >= 1 && n_rows <= 0x7fffffff - 256, "nrb_recommend: n_rows must be in [1, 2^31 - 257]");
   NRB_REQUIRE(n_users >= 1, "nrb_recommend: n_users must be >= 1");
   NRB_REQUIRE(n_excl >= 0, "nrb_recommend: n_excl must be >= 0");
+  NRB_REQUIRE(n_pool <= n_rows, "nrb_recommend: a pool of strictly ascending row ids has at most n_rows entries");
   return NRB_OK;
+}
+
+static TopkPlan rec_plan(int64_t n_users, int64_t n_rows, int64_t n_pool) {
+  return topk_plan(n_users, n_pool < 0 ? n_rows : std::max<int64_t>(n_pool, 1));
 }
 
 }  // namespace nrb
 
 using namespace nrb;
 
-extern "C" size_t nrb_recommend_workspace_bytes(int precision, int dim, int64_t n_rows, int64_t n_users,
-                                                int64_t n_excl, int k) {
-  if (check_recommend_args(precision, dim, n_rows, n_users, n_excl, k) != NRB_OK) return 0;
-  const TopkPlan plan = topk_plan(n_users, n_rows);
-  return rec_layout(nullptr, precision, dim, n_rows, n_users, n_excl, k, plan).bytes;
+extern "C" size_t nrb_recommend_pool_blend_workspace_bytes(int precision, int dim, int64_t n_rows, int64_t n_users,
+                                                           int64_t n_excl, int k, int64_t n_pool) {
+  if (check_recommend_args(precision, dim, n_rows, n_users, n_excl, k, n_pool) != NRB_OK) return 0;
+  return rec_layout(nullptr, precision, dim, n_users, n_excl, k, n_pool, rec_plan(n_users, n_rows, n_pool)).bytes;
 }
 
-extern "C" int nrb_recommend(int precision, int dim, int64_t n_rows, const void* table, int64_t table_stride,
-                             const void* table_op, int64_t op_stride, const float* users, int64_t users_stride,
-                             int64_t n_users, const int32_t* excl_idx, const int64_t* excl_off, int64_t n_excl, int k,
-                             int32_t* out_rows, float* out_scores, int32_t* err_flag, void* workspace,
-                             size_t workspace_bytes, nrb_stream_t stream) {
-  int rc = check_recommend_args(precision, dim, n_rows, n_users, n_excl, k);
+extern "C" size_t nrb_recommend_workspace_bytes(int precision, int dim, int64_t n_rows, int64_t n_users,
+                                                int64_t n_excl, int k) {
+  return nrb_recommend_pool_blend_workspace_bytes(precision, dim, n_rows, n_users, n_excl, k, -1);
+}
+
+extern "C" int nrb_recommend_pool_blend(int precision, int dim, int64_t n_rows, const void* table,
+                                        int64_t table_stride, const void* table_op, int64_t op_stride,
+                                        const float* users, int64_t users_stride, int64_t n_users,
+                                        const int32_t* excl_idx, const int64_t* excl_off, int64_t n_excl, int k,
+                                        const int32_t* pool, int64_t n_pool, const float* cand_base,
+                                        float blend_alpha, const int64_t* hist_off, int32_t* out_rows,
+                                        float* out_scores, int32_t* err_flag, void* workspace,
+                                        size_t workspace_bytes, nrb_stream_t stream) {
+  int rc = check_recommend_args(precision, dim, n_rows, n_users, n_excl, k, n_pool);
   if (rc != NRB_OK) return rc;
   NRB_REQUIRE(table && table_op && users && out_rows && out_scores && err_flag && workspace,
               "nrb_recommend: null pointer");
   NRB_REQUIRE((excl_idx == nullptr) == (excl_off == nullptr), "nrb_recommend: excl_idx and excl_off go together");
+  NRB_REQUIRE(n_pool <= 0 || pool != nullptr, "nrb_recommend: a pool of n_pool > 0 ids needs `pool`");
   NRB_REQUIRE(table_stride >= dim && users_stride >= dim && op_stride >= (precision == NRB_BF16 ? dim : 3 * dim),
               "nrb_recommend: row strides must cover the row");
-  const TopkPlan plan = topk_plan(n_users, n_rows);
-  const RecLayout L = rec_layout(workspace, precision, dim, n_rows, n_users, n_excl, k, plan);
+  NRB_REQUIRE(n_pool < 0 || (op_stride % 8 == 0 && (reinterpret_cast<uintptr_t>(table_op) & 15) == 0),
+              "nrb_recommend: with a pool, table_op must be 16-byte aligned with a 16-byte multiple row pitch");
+  const bool has_pool = n_pool >= 0;
+  const int64_t n_cols = has_pool ? n_pool : n_rows;
+  const TopkPlan plan = rec_plan(n_users, n_rows, n_pool);
+  const RecLayout L = rec_layout(workspace, precision, dim, n_users, n_excl, k, n_pool, plan);
   if (workspace_bytes < L.bytes) {
     set_error("nrb_recommend: workspace too small (%zu < %zu bytes)", workspace_bytes, L.bytes);
     return NRB_E_WORKSPACE;
@@ -268,29 +343,64 @@ extern "C" int nrb_recommend(int precision, int dim, int64_t n_rows, const void*
   const int sms = sm_count_cached();
   const int kdim = precision == NRB_BF16 ? dim : 3 * dim;
   auto warps_grid = [&](int64_t n) { return (int)std::max<int64_t>(1, std::min<int64_t>((n + 7) / 8, (int64_t)sms * 16)); };
+  auto sort_excl = [&]() -> int {
+    sort_excl_kernel<<<(unsigned)n_users, 256, 0, st>>>(excl_idx, excl_off, n_rows, has_pool ? pool : nullptr,
+                                                        n_pool, L.excl_tmp, L.excl_sorted, err_flag);
+    note_launch();
+    NRB_CUDA_CHECK(cudaGetLastError());
+    return NRB_OK;
+  };
 
+  if (n_cols == 0) {  // empty pool: nothing is eligible; excluded ids are still range-checked
+    NRB_CUDA_CHECK(cudaMemsetAsync(out_rows, 0xff, (size_t)n_users * k * sizeof(int32_t), st));  // -1
+    NRB_CUDA_CHECK(cudaMemsetAsync(out_scores, 0xff, (size_t)n_users * k * sizeof(float), st));  // NaN
+    return excl_idx != nullptr ? sort_excl() : NRB_OK;
+  }
+  const void* gemm_op = table_op;
+  int64_t gemm_ld = op_stride;
+  if (has_pool) {
+    pool_gather_kernel<<<warps_grid(n_pool), 256, 0, st>>>((const __nv_bfloat16*)table_op, op_stride, kdim, pool,
+                                                            n_pool, n_rows, (__nv_bfloat16*)L.pool_op, err_flag);
+    note_launch();
+    NRB_CUDA_CHECK(cudaGetLastError());
+    gemm_op = L.pool_op;
+    gemm_ld = kdim;
+  }
   user_operand_kernel<<<warps_grid(n_users), 256, 0, st>>>(users, users_stride, n_users, dim, precision != NRB_BF16,
-                                                           (__nv_bfloat16*)L.user_op, kdim);
+                                                           (__nv_bfloat16*)L.user_op, kdim, hist_off,
+                                                           cand_base != nullptr ? L.cold : nullptr);
   note_launch();
   NRB_CUDA_CHECK(cudaGetLastError());
   const int64_t n_pad = plan.n_per_row * 256;
-  row_scale_kernel<<<warps_grid(n_pad), 256, 0, st>>>(table, precision, table_stride, n_rows, dim, n_pad, L.scale);
+  row_scale_kernel<<<warps_grid(n_pad), 256, 0, st>>>(table, precision, table_stride, n_rows, dim,
+                                                      has_pool ? pool : nullptr, n_cols, n_pad, L.scale, cand_base,
+                                                      L.base);
   note_launch();
   NRB_CUDA_CHECK(cudaGetLastError());
   if (excl_idx != nullptr) {
-    sort_excl_kernel<<<(unsigned)n_users, 256, 0, st>>>(excl_idx, excl_off, n_rows, L.excl_tmp, L.excl_sorted,
-                                                        err_flag);
-    note_launch();
-    NRB_CUDA_CHECK(cudaGetLastError());
+    rc = sort_excl();
+    if (rc != NRB_OK) return rc;
   }
-  rc = gemm_topk_tc(L.user_op, kdim, table_op, op_stride, L.scale, excl_off, excl_idx ? L.excl_sorted : nullptr,
-                    n_users, (int)n_rows, kdim, k, plan, L.parts, st);
+  rc = gemm_topk_tc(L.user_op, kdim, gemm_op, gemm_ld, L.scale, excl_off, excl_idx ? L.excl_sorted : nullptr,
+                    n_users, (int)n_cols, kdim, k, plan, L.parts, cand_base != nullptr ? L.base : nullptr, L.cold,
+                    blend_alpha, st);
   if (rc != NRB_OK) return rc;
   const size_t merge_smem = (size_t)8 * 2 * plan.slots * sizeof(int32_t);
   if (merge_smem > 48 * 1024) NRB_CUDA_CHECK(cudaFuncSetAttribute(merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)merge_smem));
-  merge_kernel<<<(unsigned)((n_users + 7) / 8), 256, merge_smem, st>>>(L.parts, plan, n_users, k, out_rows,
+  merge_kernel<<<(unsigned)((n_users + 7) / 8), 256, merge_smem, st>>>(L.parts, plan, n_users, k,
+                                                                       has_pool ? pool : nullptr, out_rows,
                                                                        out_scores);
   note_launch();
   NRB_CUDA_CHECK(cudaGetLastError());
   return NRB_OK;
+}
+
+extern "C" int nrb_recommend(int precision, int dim, int64_t n_rows, const void* table, int64_t table_stride,
+                             const void* table_op, int64_t op_stride, const float* users, int64_t users_stride,
+                             int64_t n_users, const int32_t* excl_idx, const int64_t* excl_off, int64_t n_excl, int k,
+                             int32_t* out_rows, float* out_scores, int32_t* err_flag, void* workspace,
+                             size_t workspace_bytes, nrb_stream_t stream) {
+  return nrb_recommend_pool_blend(precision, dim, n_rows, table, table_stride, table_op, op_stride, users,
+                                  users_stride, n_users, excl_idx, excl_off, n_excl, k, nullptr, -1, nullptr, 1.0f,
+                                  nullptr, out_rows, out_scores, err_flag, workspace, workspace_bytes, stream);
 }

@@ -3,7 +3,8 @@
   get_final_attention_eval            data_model_helper.py:112-131
   get_cos_sim_scores                  data_model_helper.py:174-239
   get_final_second_attention_score    data_model_helper.py:416-443
-  get_top_k_recommendations           (new) the k best news of the whole table per user
+  get_top_k_recommendations           (new) the k best news of the table (or of a pool of it) per user, scored like
+                                      get_final_score when given the classification baseline
 
 Same positional signatures and return types (CPU tensors / numpy) as the reference; the work is
 one table upload + one dense row transform (cached per table/weights) + one fused CUDA launch
@@ -17,7 +18,7 @@ import numpy as np
 import torch
 
 from .data_utils import rank_group_preds, ranks_to_object_array
-from .engine import cached_engine
+from .engine import cached_engine, host_base, host_pool
 
 
 def get_final_attention_eval(history_rev_index: np.ndarray, history_len_list: np.ndarray,
@@ -66,17 +67,34 @@ def get_final_second_attention_score(history_rev_index: np.ndarray, history_len_
 def get_top_k_recommendations(history_rev_index: np.ndarray, history_len_list: np.ndarray,
                               news_embeddings: torch.Tensor, model: torch.nn.Module, k: int = 10,
                               exclude_history: bool = True, query_news_embeddings: Optional[torch.Tensor] = None,
-                              precision=None) -> dict:
-    """The k news of the whole table that score best against each user (no counterpart in the reference, which only
-    scores the candidate lists of the impressions).  Same user vector and cosine as `get_cos_sim_scores`; with
-    `exclude_history` a user's own history is never recommended.
+                              precision=None, pool=None, classification_score: Optional[np.ndarray] = None,
+                              weight_model=None, history_bool=None) -> dict:
+    """The k news that score best against each user (no counterpart in the reference, which only scores the candidate
+    lists of the impressions).  Same user vector and cosine as `get_cos_sim_scores`; with `exclude_history` a user's
+    own history is never recommended.
+
+    `pool` (row ids, or a bool mask over the table) restricts the news to those rows, e.g. the news of an evaluation
+    period's impressions.  With `classification_score` (one classification-head score per table row,
+    `get_classification_preds`) the score is `get_final_score`'s: sigmoid(alpha) * cosine + (1 - sigmoid(alpha)) *
+    classification score (alpha of `weight_model`; pure cosine without one), and the classification score alone for
+    users without a history.  `history_bool` (as in `get_final_score`) marks the behaviour rows that have a history;
+    `history_*` then describe those rows only, and the result has one list per behaviour row.
 
     Returns numpy {"top_k_rows": int32 [U, k] (row ids = `news_list` positions), "top_k_scores": float32 [U, k]},
     each list by score descending then row id ascending, -1 / NaN where a user has fewer than k eligible news.
     1 <= k <= 32."""
+    n_rows = news_embeddings.shape[0]
+    if history_bool is not None and classification_score is None:
+        raise ValueError("history_bool needs classification_score: users without a history are recommended by the "
+                         "classification baseline alone")
+    base = None if classification_score is None else host_base(classification_score, n_rows)
+    pool = None if pool is None else host_pool(pool, n_rows)
+    hist_len = history_len_list if history_bool is None else _full_history_lengths(history_len_list, history_bool)
+    alpha = weight_model.blend_alpha() if weight_model is not None else 1.0
     q = query_news_embeddings if isinstance(query_news_embeddings, torch.Tensor) else None
     eng = cached_engine(news_embeddings, model, q, precision=precision)
-    rows, scores = eng.recommend(history_rev_index, history_len_list, k, exclude_history=exclude_history)
+    rows, scores = eng.recommend(history_rev_index, hist_len, k, exclude_history=exclude_history, pool=pool,
+                                 cand_base=base, blend_alpha=alpha)
     return {"top_k_rows": rows.cpu().numpy(), "top_k_scores": scores.cpu().numpy()}
 
 

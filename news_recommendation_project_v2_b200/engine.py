@@ -387,14 +387,19 @@ class ScoringEngine:
         return hit[1]
 
     def recommend_device(self, hist_idx_d: torch.Tensor, hist_off_d: torch.Tensor, k: int,
-                         exclude_history: bool = True, err_flag: Optional[torch.Tensor] = None):
+                         exclude_history: bool = True, err_flag: Optional[torch.Tensor] = None,
+                         pool: Optional[torch.Tensor] = None, cand_base: Optional[torch.Tensor] = None,
+                         blend_alpha: float = 1.0):
         """Device CSR history (int32 ids, int64 offsets [U + 1]) in, the k best table rows per user out:
         (rows int32 [U, k], scores fp32 [U, k]) on the device, see `ops.recommend` for the order and padding.
 
         The user vector is the one `score` pools; its score against row r is the cosine `score` would give r as a
-        candidate.  With `exclude_history` a user's own history rows are never returned.  fp32 and fp32x3 engines
+        candidate.  With `exclude_history` a user's own history rows are never returned.  `pool` (device int32 row
+        ids, strictly ascending) restricts the rows; `cand_base` (device fp32 per table row) + `blend_alpha` blend the
+        baseline in as `score` does, users with an empty history getting the baseline alone.  fp32 and fp32x3 engines
         score on split-bf16 tensor-core operands (the FFMA GEMM has no top-k epilogue)."""
         ops._recommend_args(self.dim, k)
+        ops._recommend_pool_args(self.n_rows, hist_off_d.numel() - 1, pool, cand_base, None)
         with torch.cuda.device(self.device):
             flag = err_flag if err_flag is not None else ops.new_err_flag(self.device)
             n_imp = hist_off_d.numel() - 1
@@ -407,19 +412,27 @@ class ScoringEngine:
                 user = user[:, :self.dim].contiguous()  # drop the kernel's zero padding: logical rows and width
             excl = (hist_idx_d, hist_off_d) if exclude_history else (None, None)
             rows, scores = ops.recommend(self.cand, user, k, table_op=self._table_operand(), excl_idx=excl[0],
-                                         excl_off=excl[1], err_flag=flag)
+                                         excl_off=excl[1], err_flag=flag, pool=pool, cand_base=cand_base,
+                                         blend_alpha=blend_alpha, hist_off=hist_off_d)
             if err_flag is None:
                 ops.raise_on_index_error(flag, "recommend")
             return rows, scores
 
-    def recommend(self, hist_idx, hist_len, k: int, exclude_history: bool = True):
-        """Host history arrays (`history_rev_ind_array[0]`, `history_len_list`) in: the k best rows of the whole
-        table for each user, (rows int32 [U, k], scores fp32 [U, k]) on the device."""
+    def recommend(self, hist_idx, hist_len, k: int, exclude_history: bool = True, pool=None, cand_base=None,
+                  blend_alpha: float = 1.0):
+        """Host history arrays (`history_rev_ind_array[0]`, `history_len_list`) in: the k best rows of the table for
+        each user, (rows int32 [U, k], scores fp32 [U, k]) on the device.  `pool`: host row ids (any order,
+        duplicates allowed) or a bool mask over the table, see `host_pool`; `cand_base`: fp32 per table row."""
         ops._recommend_args(self.dim, k)
+        pool_np = None if pool is None else host_pool(pool, self.n_rows)
+        base_np = None if cand_base is None else host_base(cand_base, self.n_rows)
         with torch.cuda.device(self.device):
             h_off, n_h = _offsets(hist_len, self.device)
             assert n_h == len(hist_idx), "history index length should match history_len_list"
-            return self.recommend_device(_as_i32(hist_idx, self.device), h_off, k, exclude_history=exclude_history)
+            pool_d = None if pool_np is None else torch.from_numpy(pool_np).to(self.device)
+            base_d = None if base_np is None else torch.from_numpy(base_np).to(self.device)
+            return self.recommend_device(_as_i32(hist_idx, self.device), h_off, k, exclude_history=exclude_history,
+                                         pool=pool_d, cand_base=base_d, blend_alpha=blend_alpha)
 
     def user_vectors(self, hist_idx, hist_len) -> torch.Tensor:
         """get_final_attention_eval: fp32 [I, d] user vectors (device)."""
@@ -434,6 +447,30 @@ class ScoringEngine:
                                         _as_i32(hist_idx, self.device), h_off, empty, zeros, 0, want_user=True,
                                         want_ranks=False)
             return user if user.shape[1] == self.cand.shape[1] else user[:, :self.cand.shape[1]].contiguous()
+
+
+def host_pool(pool, n_rows: int) -> np.ndarray:
+    """A host pool as `ops.recommend` takes it: a bool mask over the n_rows table rows -> the rows it selects, or row
+    ids in any order with duplicates -> the distinct ids ascending (int32).  Ids outside [0, n_rows) raise IndexError."""
+    p = np.asarray(pool)
+    if p.dtype == np.bool_:
+        if p.shape != (n_rows,):
+            raise ValueError(f"a boolean pool must be a mask over the {n_rows} table rows, got shape {p.shape}")
+        return np.flatnonzero(p).astype(np.int32)
+    if p.ndim != 1 or (p.size and not np.issubdtype(p.dtype, np.integer)):
+        raise ValueError("a pool must be a 1-D array of integer row ids or a boolean mask")
+    ids = np.unique(p.astype(np.int64))
+    if ids.size and (ids[0] < 0 or ids[-1] >= n_rows):
+        raise IndexError(f"pool: row id out of range for a table of {n_rows} rows")
+    return ids.astype(np.int32)
+
+
+def host_base(cand_base, n_rows: int) -> np.ndarray:
+    """A host per-row baseline (one fp32 score per table row, e.g. `get_classification_preds`)."""
+    b = np.ascontiguousarray(np.asarray(cand_base, dtype=np.float32))
+    if b.shape != (n_rows,):
+        raise ValueError(f"the baseline must have one score per table row ({n_rows}), got shape {b.shape}")
+    return b
 
 
 _engine_cache: dict = {}

@@ -205,22 +205,52 @@ def _recommend_args(dim: int, k: int) -> None:
         raise _lib.NrbError(f"recommend: the embedding width must be a multiple of 64 (got {dim})")
 
 
+def _recommend_pool_args(n_rows: int, n_users: int, pool, cand_base, hist_off) -> None:
+    """dtype and shape checks of the pool / baseline / history arguments of `recommend`, before any device work."""
+    if pool is not None:
+        if not isinstance(pool, torch.Tensor) or pool.dtype != torch.int32 or pool.dim() != 1:
+            raise _lib.NrbError("recommend: pool must be a 1-D int32 tensor of table row ids")
+        if pool.numel() > n_rows:
+            raise _lib.NrbError(f"recommend: a pool of distinct row ids has at most {n_rows} entries")
+    if cand_base is not None:
+        if not isinstance(cand_base, torch.Tensor) or cand_base.dtype != torch.float32 or cand_base.dim() != 1:
+            raise _lib.NrbError("recommend: cand_base must be a 1-D float32 tensor")
+        if cand_base.numel() != n_rows:
+            raise _lib.NrbError(f"recommend: cand_base must have one entry per table row ({n_rows})")
+    if hist_off is not None:
+        if not isinstance(hist_off, torch.Tensor) or hist_off.dtype != torch.int64 or hist_off.dim() != 1:
+            raise _lib.NrbError("recommend: hist_off must be a 1-D int64 tensor")
+        if hist_off.numel() != n_users + 1:
+            raise _lib.NrbError("recommend: hist_off must have U + 1 entries")
+
+
 def recommend(table: torch.Tensor, users: torch.Tensor, k: int, table_op: Optional[torch.Tensor] = None,
               excl_idx: Optional[torch.Tensor] = None, excl_off: Optional[torch.Tensor] = None,
-              err_flag: Optional[torch.Tensor] = None):
-    """The k best rows of the whole table for each user (nrb_recommend): (rows int32 [U, k], scores fp32 [U, k]).
+              err_flag: Optional[torch.Tensor] = None, pool: Optional[torch.Tensor] = None,
+              cand_base: Optional[torch.Tensor] = None, blend_alpha: float = 1.0,
+              hist_off: Optional[torch.Tensor] = None):
+    """The k best rows of the table for each user (nrb_recommend_pool_blend): (rows int32 [U, k], scores fp32 [U, k]).
 
     score = cosine(user, row), ordered by score descending then row id ascending, (-1, NaN) once a user has no
     eligible rows left.  bf16 tables run the tensor-core GEMM on bf16 operands; fp32 tables run it on split-bf16
     operands (`table_op` = split_rows(table, 1), built here if not given).  The fp32 FFMA GEMM has no top-k epilogue,
     so fp32 retrieval always uses the split tensor-core path.  `excl_idx` / `excl_off` (int32 ids, int64 offsets
-    [U + 1]): rows never returned for each user; an out-of-range id raises IndexError (or sets bit 0 of `err_flag`)."""
+    [U + 1]): rows never returned for each user; an out-of-range id raises IndexError (or sets bit 0 of `err_flag`).
+
+    `pool` (device int32 row ids, strictly ascending): only these rows are eligible and the GEMM runs over them alone;
+    returned ids stay table row ids.  Ids out of range or not ascending raise IndexError like `excl_idx`.
+    `cand_base` (device fp32 [N]) + `blend_alpha`: score = cos * alpha + base * (1 - alpha), or base alone for users
+    whose history is empty in `hist_off` (device int64 [U + 1]; None: every user has a history) -- the blend and the
+    fallback of `score_rank`.  NaN scores are never returned."""
     _recommend_args(table.shape[1] if table.dim() == 2 else 0, k)
+    if users.dim() != 2:
+        raise _lib.NrbError("users must be [U, d]")
+    _recommend_pool_args(table.shape[0] if table.dim() == 2 else 0, users.shape[0], pool, cand_base, hist_off)
     dev = require_device(table.device)
     _dev(table, "table")
     _dev(users, "users", torch.float32)
     n_rows, dim = table.shape
-    if users.dim() != 2 or users.shape[1] != dim:
+    if users.shape[1] != dim:
         raise _lib.NrbError(f"users must be [U, {dim}]")
     prec = dtype_code(table.dtype)
     if table_op is None:
@@ -235,20 +265,28 @@ def recommend(table: torch.Tensor, users: torch.Tensor, k: int, table_op: Option
         if excl_off.numel() != users.shape[0] + 1:
             raise _lib.NrbError("excl_off must have U + 1 entries")
         n_excl = excl_idx.numel()
+        if n_excl == 0:  # an empty id tensor may have no storage (NULL): nothing is excluded
+            excl_idx = excl_off = None
+    for t, n in ((pool, "pool"), (cand_base, "cand_base"), (hist_off, "hist_off")):
+        if t is not None:
+            _dev(t, n)
+    n_pool = -1 if pool is None else pool.numel()
     U = users.shape[0]
     rows = torch.empty(U, k, dtype=torch.int32, device=dev)
     scores = torch.empty(U, k, dtype=torch.float32, device=dev)
     if U == 0:
         return rows, scores
     lib = load()
-    ws_bytes = lib.nrb_recommend_workspace_bytes(prec, dim, n_rows, U, n_excl, int(k))
+    ws_bytes = lib.nrb_recommend_pool_blend_workspace_bytes(prec, dim, n_rows, U, n_excl, int(k), n_pool)
     if ws_bytes == 0:
-        check(-1, "nrb_recommend_workspace_bytes")
+        check(-1, "nrb_recommend_pool_blend_workspace_bytes")
     ws = _workspace(dev, ws_bytes, "recommend")
     flag = err_flag if err_flag is not None else new_err_flag(dev)
-    check(lib.nrb_recommend(prec, dim, n_rows, ptr(table), table.stride(0), ptr(table_op), table_op.stride(0),
-                            ptr(users), users.stride(0), U, ptr(excl_idx), ptr(excl_off), n_excl, int(k), ptr(rows),
-                            ptr(scores), ptr(flag), ptr(ws), ws.numel(), stream_ptr()), "nrb_recommend")
+    check(lib.nrb_recommend_pool_blend(prec, dim, n_rows, ptr(table), table.stride(0), ptr(table_op),
+                                       table_op.stride(0), ptr(users), users.stride(0), U, ptr(excl_idx),
+                                       ptr(excl_off), n_excl, int(k), ptr(pool), n_pool, ptr(cand_base),
+                                       float(blend_alpha), ptr(hist_off), ptr(rows), ptr(scores), ptr(flag), ptr(ws),
+                                       ws.numel(), stream_ptr()), "nrb_recommend_pool_blend")
     if err_flag is None:
         raise_on_index_error(flag, "recommend")
     return rows, scores

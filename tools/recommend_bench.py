@@ -1,6 +1,7 @@
-"""Whole-table retrieval at MIND-large scale: fused tensor-core GEMM + top-k (nrb_recommend) vs the unfused path.
+"""Whole-table retrieval at MIND-large scale: fused tensor-core GEMM + top-k (nrb_recommend) vs the unfused path, and
+retrieval from a pool with the classification-baseline blend (nrb_recommend_pool_blend).
 
-    python tools/recommend_bench.py [--users 65536] [--ks 10,32] [--iters 5] [--out FILE]
+    python tools/recommend_bench.py [--users 65536] [--ks 10,32] [--iters 5] [--pool-k 10] [--out FILE]
 
 Workload: the MIND-large table (161,013 x 1024, bf16, synthetic FinalAttention weights as in bench.py), U users with
 bench.py's history distribution (H ~ clip(Geom(1/32), 1, 50)), history excluded.  Per k it reports, from CUDA events
@@ -11,6 +12,11 @@ after warm-up:
     MEASURED_PEAKS.json (bench.py's fallback figure when the file is absent);
   * the unfused path in the same process: nrb_linear to fp32 scores in user chunks, scale by the row norms, mask
     history, torch.topk; its time and the number of users whose row lists differ from the fused result.
+Then, at k = --pool-k, four legs of the fused call timed back to back in the same process ("pool_blend"): plain,
+pool = a random N/8 of the rows, blend (baseline for every row, alpha 0.7, the bench's users all have a history), and
+pool + blend; each with ms per call and the executed TFLOP/s of the call, 2 U n_pool d / t (n_pool = N without a
+pool).  The legs run after each other in rounds (plain, pool, blend, pool + blend, repeated --rounds times) and report
+the median, so that a drift of the clocks over the run reaches every leg alike.
 The GPU name and power limit come from a read-only nvidia-smi query in the same run.  Needs a B200.
 """
 from __future__ import annotations
@@ -87,11 +93,40 @@ def kernel_split(fn) -> dict:
         name = ev.name
         key = ("gemm_topk" if "gemm_tc_kernel" in name else "merge" if "merge_kernel" in name else
                "user_operand" if "user_operand" in name else "row_norms" if "row_scale" in name else
-               "history_sort" if "sort_excl" in name else None)
+               "history_sort" if "sort_excl" in name else "pool_gather" if "pool_gather" in name else None)
         if key is None:
             continue
         out[key] = out.get(key, 0.0) + ev.device_time / 1000.0
     return {k: round(v, 4) for k, v in out.items()}
+
+
+def pool_blend_legs(eng, user, hist_idx, h_off, k, iters, warmup, rounds, flag) -> dict:
+    """ms per call and executed TFLOP/s of plain / pool N/8 / blend / pool + blend, alternated over `rounds`."""
+    n_rows, d = eng.cand.shape
+    U = user.shape[0]
+    g = torch.Generator(device=user.device).manual_seed(99)
+    pool = torch.sort(torch.randperm(n_rows, generator=g, device=user.device)[:n_rows // 8])[0].to(torch.int32)
+    base = torch.rand(n_rows, generator=g, device=user.device)  # a classification probability per row
+    legs = {"plain": {}, "pool_n_over_8": dict(pool=pool), "blend": dict(cand_base=base, blend_alpha=0.7),
+            "pool_n_over_8_blend": dict(pool=pool, cand_base=base, blend_alpha=0.7)}
+    fns = {name: (lambda kw=kw: ops.recommend(eng.cand, user, k, excl_idx=hist_idx, excl_off=h_off, err_flag=flag,
+                                               hist_off=h_off, **kw)) for name, kw in legs.items()}
+    for fn in fns.values():
+        for _ in range(warmup):
+            fn()
+    times = {name: [] for name in fns}
+    for _ in range(rounds):
+        for name, fn in fns.items():
+            times[name].append(timed(fn, iters))
+    out = {"k": k, "n_pool": int(pool.numel()), "rounds": rounds, "iters_per_round": iters, "legs": {}}
+    for name, ts in times.items():
+        t = sorted(ts)[len(ts) // 2]
+        cols = int(pool.numel()) if "pool" in legs[name] else n_rows
+        out["legs"][name] = {"ms": round(t, 4), "ms_all_rounds": [round(x, 4) for x in ts],
+                             "tflops": round(2.0 * U * cols * d / (t * 1e-3) / 1e12, 1),
+                             "kernels_ms": kernel_split(fns[name])}
+        print(f"pool/blend k={k} {name}: {t:.3f} ms, {out['legs'][name]['tflops']} TFLOP/s", file=sys.stderr)
+    return out
 
 
 def main():
@@ -101,6 +136,8 @@ def main():
     ap.add_argument("--iters", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--chunk", type=int, default=4096, help="users per unfused GEMM chunk")
+    ap.add_argument("--pool-k", type=int, default=10, help="k of the pool / blend legs")
+    ap.add_argument("--rounds", type=int, default=5, help="rounds over the pool / blend legs")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
 
@@ -176,6 +213,7 @@ def main():
         }
         print(f"k={k}: fused {t_fused:.3f} ms {split}, unfused {t_unf:.3f} ms, lists differ for {diff_rows} users",
               file=sys.stderr)
+    results["pool_blend"] = pool_blend_legs(eng, user, hist_idx, h_off, a.pool_k, a.iters, a.warmup, a.rounds, flag)
     ops.raise_on_index_error(flag, "recommend_bench")
     line = json.dumps(results)
     print(line)
