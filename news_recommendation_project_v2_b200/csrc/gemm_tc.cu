@@ -30,7 +30,6 @@
 #include "ptx.cuh"
 
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 namespace nrb {
@@ -95,17 +94,19 @@ struct GemmParams {
   int group_valid;  // softmax: valid columns per group (L <= Lp)
   int cluster;      // softmax: CTAs per cluster = max(1, Lp / 256)
   PushJob push;     // rows of an earlier result that the spare warp multicasts to every rank while the GEMM runs
-  // NRB_EPI_TOPK reuses fields (the parameter block of every other instantiation stays as it is):
-  //   bias    = per-column scale 1 / max(|w_n|, 1e-8), NaN from column N up to the next multiple of 256
-  //   res     = int64 CSR offsets [M + 1] of the excluded columns of each row (NULL: nothing excluded)
-  //   res_map = the excluded columns, sorted ascending within each row
-  //   y       = partial lists, 8-byte (score, column) entries [rows][2 halves][ldy slots][group]
-  //   ldy     = slots per (row, half): CTAs (pairs) whose contiguous unit range touches one row block
-  //   group   = k
-  // NRB_EPI_TOPK_BLEND adds (appended, so that the offsets of every other field stay as they are):
-  const float* topk_base;    // per-column baseline, NaN from column N up to the next multiple of 256
-  const uint8_t* topk_cold;  // per row: 1 = empty history, the score is topk_base alone
-  float topk_alpha;          // score = acc * scale * alpha + base * (1 - alpha) for the other rows
+  // NRB_EPI_TOPK / NRB_EPI_TOPK_BLEND, which read no other field but the shape (placed last, so that the parameter
+  // offsets of every other epilogue stay as they are)
+  struct TopkArgs {
+    const float* scale;          // per-column 1 / max(|w_n|, 1e-8), NaN from column N up to the next multiple of 256
+    const int64_t* excl_off;     // CSR offsets [M + 1] of the excluded columns of each row (NULL: nothing excluded)
+    const int32_t* excl_sorted;  // the excluded columns, sorted ascending within each row
+    uint2* parts;                // partial lists, 8-byte (score, column) entries [rows][2 halves][slots][k]
+    int64_t slots;               // per (row, half): CTAs (pairs) whose contiguous unit range touches one row block
+    int k;
+    const float* base;           // blend: per-column baseline, NaN from column N up to the next multiple of 256
+    const uint8_t* cold;         // blend: per row, 1 = empty history, the score is base alone
+    float alpha;                 // blend: score = acc * scale * alpha + base * (1 - alpha) for the other rows
+  } topk;
 };
 
 __device__ __forceinline__ float ex2_approx(float x) {
@@ -259,6 +260,63 @@ __device__ __forceinline__ void stage_values(uint32_t base, int r, int j0, const
                  pack_bf16x2(v[8 * q + 6], v[8 * q + 7]));
 }
 
+// Position in a ring of N mbarrier-guarded buffers, and the parity of the pass over the ring it is in
+template <int N>
+struct Ring {
+  int i = 0;
+  uint32_t phase = 0;
+  __device__ __forceinline__ void advance() {
+    if (++i == N) {
+      i = 0;
+      phase ^= 1;
+    }
+  }
+};
+
+// The 4 x 32-column accumulator chunks of this warp's half (TMEM address taddr), each loaded while the one before it
+// is worked on:
+//   TmemChunks ch(taddr);
+//   #pragma unroll
+//   for (int c = 0; c < 4; ++c) { const uint32_t(&r)[32] = ch.wait(c, release); ... }
+// wait(c) returns chunk c and starts the load of chunk c + 1.  release() runs once the last load has completed, before
+// the last chunk's math: with it the epilogue hands the accumulator back to the MMA warp as early as it can.  (The
+// loop body stays in the caller: as a lambda, the top-k body compiled to more registers and a longer insertion path.)
+struct TmemChunks {
+  uint32_t taddr;
+  uint32_t rbuf[2][32];
+  __device__ __forceinline__ explicit TmemChunks(uint32_t a) : taddr(a) { ptx::tmem_ld_32x32(taddr, rbuf[0]); }
+  template <typename Release>
+  __device__ __forceinline__ const uint32_t (&wait(int c, Release release))[32] {
+    ptx::tmem_ld_wait();
+    if (c + 1 < 4) ptx::tmem_ld_32x32(taddr + (uint32_t)((c + 1) * 32), rbuf[(c + 1) & 1]);  // prefetch
+    if (c == 3) release();
+    return rbuf[c & 1];
+  }
+};
+
+// One epilogue half's two 128-row x 64-column bf16 staging buffers, filled in turn ("groups") by the half's 4 warps
+// and written out by TMA stores of the half's first thread.
+struct StoreGroups {
+  uint8_t* base;
+  int bar_id;  // named barrier of the half (128 threads)
+  bool issuer;
+  uint32_t gsel = 0;  // buffer of the current group
+  __device__ __forceinline__ uint8_t* buf() const { return base + gsel * kGroupBytes; }
+  __device__ __forceinline__ void begin() {  // the buffer used two groups ago must be drained
+    if (issuer) ptx::tma_store_wait_read1();
+    ptx::named_bar_sync(bar_id, 128);
+  }
+  __device__ __forceinline__ void end(const CUtensorMap* map, bool store, int col, int row) {
+    ptx::fence_proxy_async();
+    ptx::named_bar_sync(bar_id, 128);
+    if (issuer) {
+      if (store) ptx::tma_store_2d(map, buf(), col, row);
+      ptx::tma_store_commit();  // committed even when empty: keeps the group count in step with gsel
+    }
+    gsel ^= 1;
+  }
+};
+
 template <int BN, int EPI, bool OUT_BF16, int CG>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_w,
@@ -292,23 +350,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   const bool clustered = CS > 1 || CG == 2;
   const uint32_t cta_rank = clustered ? ptx::cluster_ctarank() : 0;
   const uint32_t unit = clustered ? ptx::cluster_id_x() : blockIdx.x;  // scheduling unit = cluster
-  const uint32_t n_units = clustered ? ptx::num_clusters_x() : gridDim.x;
 
   const int64_t M = p.m_dev != nullptr ? min(p.M, (int64_t)*p.m_dev) : p.M;
-  const int m_tiles = (int)((M + kBM * CG - 1) / (kBM * CG));  // row blocks per scheduling unit: 128*CG rows
-  const int n_tiles = (p.N + BN - 1) / BN;
-  const int n_units_per_row = n_tiles / CS;  // host guarantees n_tiles % CS == 0
-  const int64_t total_units = (int64_t)m_tiles * n_units_per_row;
+  const TileSchedule sched(M, p.N, BN, CG, CS, clustered ? ptx::num_clusters_x() : gridDim.x);
   const int k_blocks = p.K / kBK;
-  // Units are strided over the grid (u = unit, unit + n_units, ...), except for the top-k epilogue: there each unit
-  // takes one contiguous range, row block by row block with N tiles ascending, so that a thread's list lives across
-  // all the tiles its CTA does for one row block and is written out once per (row block, CTA).
-  int64_t u_first = unit, u_last = total_units, u_step = n_units;
-  if constexpr (Cfg::kTopk) {
-    u_first = (int64_t)unit * total_units / n_units;
-    u_last = ((int64_t)unit + 1) * total_units / n_units;
-    u_step = 1;
-  }
+  // top-k: each CTA (pair) takes one contiguous range, so that a thread's list lives across all the tiles its CTA
+  // does for one row block and is written out once per (row block, CTA)
+  const int64_t u_first = sched.first(unit, Cfg::kTopk), u_last = sched.end(unit, Cfg::kTopk);
+  const int64_t u_step = sched.step(Cfg::kTopk);
 
   if (warp == 0 && lane == 0) {
     ptx::prefetch_tensormap(&map_a);
@@ -328,13 +377,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     ptx::fence_barrier_init();
   }
   if (warp == 2) {
-    if (CG == 2) {
-      ptx::tmem_alloc_cg2(tmem_slot, Cfg::kTmemCols);
-      ptx::tmem_relinquish_cg2();
-    } else {
-      ptx::tmem_alloc(tmem_slot, Cfg::kTmemCols);
-      ptx::tmem_relinquish();
-    }
+    ptx::tmem_alloc<CG>(tmem_slot, Cfg::kTmemCols);
+    ptx::tmem_relinquish<CG>();
   }
   ptx::tc_fence_before();
   __syncthreads();
@@ -345,35 +389,19 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   if (warp == 0) {
     // ===================== TMA producer =====================
     if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
+      Ring<kStages> s;
       for (int64_t u = u_first; u < u_last; u += u_step) {
-        const int m_blk = (int)(u / n_units_per_row) * CG + (CG == 2 ? (int)cta_rank : 0);
-        const int n_blk = (int)(u % n_units_per_row) * CS + (CG == 2 ? 0 : (int)cta_rank);
+        const int m_blk = sched.m_blk(u, cta_rank), n_blk = sched.n_blk(u, cta_rank);
         for (int kb = 0; kb < k_blocks; ++kb) {
-          ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
-          if (CG == 2) {
-            // both CTAs fill their own smem; all bytes are counted on the LEADER's barrier
-            const uint32_t lbar = ptx::leader_addr(ptx::smem_u32(&full_bar[stage]));
-            // (the peer's bytes can only be issued after the stage's previous phase completed, so they are
-            //  always accounted to the right phase even if they land before the leader's expect_tx)
-            if (cta_rank == 0) ptx::mbar_expect_tx(&full_bar[stage], 2 * Cfg::kStageBytes);
-            ptx::tma_load_2d_cg2(smem_a + stage * Cfg::kABytes, &map_a, lbar, kb * kBK, m_blk * kBM);
-            ptx::tma_load_2d_cg2(smem_b + stage * Cfg::kBBytes, &map_w, lbar, kb * kBK,
-                                 n_blk * BN + (int)cta_rank * (BN / 2));
-            if (++stage == kStages) {
-              stage = 0;
-              phase ^= 1;
-            }
-            continue;
-          }
-          ptx::mbar_expect_tx(&full_bar[stage], Cfg::kStageBytes);
-          ptx::tma_load_2d(smem_a + stage * Cfg::kABytes, &map_a, &full_bar[stage], kb * kBK, m_blk * kBM);
-          ptx::tma_load_2d(smem_b + stage * Cfg::kBBytes, &map_w, &full_bar[stage], kb * kBK, n_blk * BN);
-          if (++stage == kStages) {
-            stage = 0;
-            phase ^= 1;
-          }
+          ptx::mbar_wait(&empty_bar[s.i], s.phase ^ 1);
+          // a pair counts both CTAs' bytes on the LEADER's barrier (the peer's bytes can only be issued after the
+          // stage's previous phase completed, so they are always accounted to the right phase even if they land
+          // before the leader's expect_tx); each CTA loads its A tile and its 1 / CG of the W tile
+          if (CG == 1 || cta_rank == 0) ptx::mbar_expect_tx(&full_bar[s.i], CG * Cfg::kStageBytes);
+          ptx::tma_load_2d<CG>(smem_a + s.i * Cfg::kABytes, &map_a, &full_bar[s.i], kb * kBK, m_blk * kBM);
+          ptx::tma_load_2d<CG>(smem_b + s.i * Cfg::kBBytes, &map_w, &full_bar[s.i], kb * kBK,
+                               n_blk * BN + (CG == 2 ? (int)cta_rank * (BN / 2) : 0));
+          s.advance();
         }
       }
     }
@@ -381,46 +409,28 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     // ===================== MMA issuer =====================
     if (lane == 0 && (CG == 1 || cta_rank == 0)) {  // pair: only the leader CTA issues
       constexpr uint32_t idesc = ptx::make_idesc_bf16(kBM * CG, BN);
-      int stage = 0;
-      uint32_t phase = 0;
-      int acc = 0;
-      uint32_t acc_phase = 0;
+      Ring<kStages> s;
+      Ring<2> acc;
       for (int64_t u = u_first; u < u_last; u += u_step) {
-        ptx::mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
+        ptx::mbar_wait(&tmem_empty[acc.i], acc.phase ^ 1);
         ptx::tc_fence_after();
-        const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BN);
+        const uint32_t tmem_d = tmem_base + (uint32_t)(acc.i * BN);
         for (int kb = 0; kb < k_blocks; ++kb) {
-          ptx::mbar_wait(&full_bar[stage], phase);
+          ptx::mbar_wait(&full_bar[s.i], s.phase);
           ptx::tc_fence_after();
-          const uint32_t a_addr = ptx::smem_u32(smem_a + stage * Cfg::kABytes);
-          const uint32_t b_addr = ptx::smem_u32(smem_b + stage * Cfg::kBBytes);
+          const uint32_t a_addr = ptx::smem_u32(smem_a + s.i * Cfg::kABytes);
+          const uint32_t b_addr = ptx::smem_u32(smem_b + s.i * Cfg::kBBytes);
 #pragma unroll
           for (int k = 0; k < kBK / kUmmaK; ++k) {
             const uint64_t da = ptx::make_smem_desc_sw128(a_addr + k * kUmmaK * 2);
             const uint64_t db = ptx::make_smem_desc_sw128(b_addr + k * kUmmaK * 2);
-            if (CG == 2)
-              ptx::mma_bf16_ss_cg2(tmem_d, da, db, idesc, (kb | k) != 0 ? 1u : 0u);
-            else
-              ptx::mma_bf16_ss(tmem_d, da, db, idesc, (kb | k) != 0 ? 1u : 0u);
+            ptx::mma_bf16_ss<CG>(tmem_d, da, db, idesc, (kb | k) != 0 ? 1u : 0u);
           }
-          // smem stage reusable once these MMAs retire (pair: signalled in both CTAs)
-          if (CG == 2)
-            ptx::mma_commit_cg2(&empty_bar[stage]);
-          else
-            ptx::mma_commit(&empty_bar[stage]);
-          if (++stage == kStages) {
-            stage = 0;
-            phase ^= 1;
-          }
+          ptx::mma_commit<CG>(&empty_bar[s.i]);  // smem stage reusable once these MMAs retire (pair: in both CTAs)
+          s.advance();
         }
-        if (CG == 2)
-          ptx::mma_commit_cg2(&tmem_full[acc]);  // accumulator complete (both CTAs' epilogues)
-        else
-          ptx::mma_commit(&tmem_full[acc]);
-        if (++acc == 2) {
-          acc = 0;
-          acc_phase ^= 1;
-        }
+        ptx::mma_commit<CG>(&tmem_full[acc.i]);  // accumulator complete (pair: both CTAs' epilogues)
+        acc.advance();
       }
     }
   } else if (warp == 3) {
@@ -433,33 +443,33 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     const int hf = e >> 2;   // which 128-column half of the accumulator tile
     const int r_tile = quad * 32 + lane;
     const bool issuer = (quad == 0 && lane == 0);
-    const int bar_id = 1 + hf;  // named barrier of this half (128 threads)
-    uint8_t* const stg_base = staging + hf * 2 * kGroupBytes;  // this half's two staging buffers
-    uint32_t gsel = 0;                                           // which of the two the next group uses
-    int acc = 0;
-    uint32_t acc_phase = 0;
+    StoreGroups out{staging + hf * 2 * kGroupBytes, 1 + hf, issuer};
+    Ring<2> acc;
     uint32_t it = 0;
     int topk_cnt = 0;            // top-k: entries in this thread's list
     float topk_thr = -INFINITY;  // top-k: score a column must beat (the k-th best once the list is full)
     int64_t hcur = 0, hend = 0;  // top-k: cursor into this row's sorted excluded columns
     bool topk_cold = false;      // top-k blend: this row scores by the baseline alone
     // accumulator hand-back: the (leader's) MMA warp waits for every epilogue warp of the pair
-    auto release_tmem = [&](int a) {
-      // (TMEM reads are ordered by tcgen05.fence::before_thread_sync; no memory release is needed, which
-      //  spares the peer CTA a cluster-scope MEMBAR per tile)
-      if (CG == 2 && cta_rank != 0)
-        ptx::mbar_arrive_cluster_relaxed(ptx::leader_addr(ptx::smem_u32(&tmem_empty[a])));
-      else
-        ptx::mbar_arrive(&tmem_empty[a]);
+    // (TMEM reads are ordered by tcgen05.fence::before_thread_sync; no memory release is needed, which spares the
+    //  peer CTA a cluster-scope MEMBAR per tile)
+    auto release_tmem = [&] {
+      ptx::tc_fence_before();
+      __syncwarp();
+      if (lane == 0) {
+        if (CG == 2 && cta_rank != 0)
+          ptx::mbar_arrive_cluster_relaxed(ptx::leader_addr(ptx::smem_u32(&tmem_empty[acc.i])));
+        else
+          ptx::mbar_arrive(&tmem_empty[acc.i]);
+      }
     };
     for (int64_t u = u_first; u < u_last; u += u_step, ++it) {
-      const int m_blk = (int)(u / n_units_per_row) * CG + (CG == 2 ? (int)cta_rank : 0);
-      const int n_blk = (int)(u % n_units_per_row) * CS + (CG == 2 ? 0 : (int)cta_rank);
-      ptx::mbar_wait(&tmem_full[acc], acc_phase);
+      const int m_blk = sched.m_blk(u, cta_rank), n_blk = sched.n_blk(u, cta_rank);
+      ptx::mbar_wait(&tmem_full[acc.i], acc.phase);
       ptx::tc_fence_after();
       const int64_t row = (int64_t)m_blk * kBM + r_tile;
       const bool row_ok = row < M;
-      const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BN + hf * 128);
+      const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc.i * BN + hf * 128);
       const int colh = n_blk * BN + hf * 128;  // first accumulator column of this half
 
       if constexpr (Cfg::kSoftmax) {
@@ -473,13 +483,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         const bool masked = lv < lp;
         const bool half_ok = colh < p.N;
         float mx[4], sm[4], mcb[4];  // group max / sum, chunk-local max * log2e
-        uint32_t rbuf[2][32];
-        ptx::tmem_ld_32x32(taddr, rbuf[0]);
+        TmemChunks pass_a(taddr);
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
-          ptx::tmem_ld_wait();
-          if (c + 1 < 4) ptx::tmem_ld_32x32(taddr + (uint32_t)((c + 1) * 32), rbuf[(c + 1) & 1]);  // prefetch
-          const uint32_t(&r)[32] = rbuf[c & 1];
+          const uint32_t(&r)[32] = pass_a.wait(c, [] {});
           float xv[32];
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
@@ -561,17 +568,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           mx[0] = mx[1] = mx[2] = mx[3] = m;
           sm[0] = sm[1] = sm[2] = sm[3] = st;
         }
-        ptx::tmem_ld_32x32(taddr, rbuf[0]);
+        TmemChunks pass_b(taddr);
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
-          ptx::tmem_ld_wait();
-          if (c + 1 < 4) ptx::tmem_ld_32x32(taddr + (uint32_t)((c + 1) * 32), rbuf[(c + 1) & 1]);  // prefetch
-          const uint32_t(&r)[32] = rbuf[c & 1];
-          if (c == 3) {  // accumulator fully consumed: hand the TMEM buffer back to the MMA warp
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) release_tmem(acc);
-          }
+          const uint32_t(&r)[32] = pass_b.wait(c, release_tmem);
           // p = exp(x - m_c) * 2^((m_c - M) log2e) / S   (masked columns already hold exp(-inf) = 0; a chunk with
           // no valid column has m_c = -inf, so its factor is 2^-inf = 0)
           const float f = ex2_approx(mcb[c] - mx[c] * kLog2e) / sm[c];
@@ -580,38 +580,25 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 #pragma unroll
           for (int j = 0; j < 32; j += 2)
             unpack2(mul2(pack2(__uint_as_float(r[j]), __uint_as_float(r[j + 1])), f2), v[j], v[j + 1]);
-          if ((c & 1) == 0) {  // first chunk of a group: the buffer used two groups ago must be drained
-            if (issuer) ptx::tma_store_wait_read1();
-            ptx::named_bar_sync(bar_id, 128);
-          }
-          stage_values<32>(ptx::smem_u32(stg_base + gsel * kGroupBytes), r_tile, (c & 1) * 4, v);
-          if ((c & 1) == 1) {
-            ptx::fence_proxy_async();
-            ptx::named_bar_sync(bar_id, 128);
-            if (issuer) {
-              if (half_ok) ptx::tma_store_2d(&map_y, stg_base + gsel * kGroupBytes, colh + (c >> 1) * 64, m_blk * kBM);
-              ptx::tma_store_commit();  // committed even when empty: keeps the group count in step with gsel
-            }
-            gsel ^= 1;
-          }
+          if ((c & 1) == 0) out.begin();
+          stage_values<32>(ptx::smem_u32(out.buf()), r_tile, (c & 1) * 4, v);
+          if ((c & 1) == 1) out.end(&map_y, half_ok, colh + (c >> 1) * 64, m_blk * kBM);
         }
       } else if constexpr (Cfg::kTopk) {
         // ---------- top-k: score = acc * scale[col]; columns that beat the k-th best enter a smem list ----------
         // (blend: score = cold ? base[col] : acc * scale[col] * alpha + base[col] * (1 - alpha), a select so that a
         //  NaN user vector of an empty history cannot reach the list)
-        const int k = p.group;
-        const int64_t m_u = u / n_units_per_row;  // row block of the unit
+        const int k = p.topk.k;
         uint2* const list = topk_list + (e * 32 + lane);
         constexpr int kLs = kEpiWarps * 32;  // stride between a thread's entries (conflict-free: lane-contiguous)
-        const int32_t* const hist = p.res_map;
-        if (u == u_first || u % n_units_per_row == 0) {  // a row-block segment starts: empty list, cursor to colh
+        const int32_t* const hist = p.topk.excl_sorted;
+        if (sched.starts_segment(u, u_first)) {  // a row-block segment starts: empty list, cursor to colh
           topk_cnt = 0;
           topk_thr = -INFINITY;
           hcur = hend = 0;
-          if constexpr (Cfg::kBlend) topk_cold = row_ok && p.topk_cold[row] != 0;
-          if (p.res != nullptr && row_ok) {
-            const int64_t* ho = reinterpret_cast<const int64_t*>(p.res);
-            int64_t lo = ho[row], hi = ho[row + 1];
+          if constexpr (Cfg::kBlend) topk_cold = row_ok && p.topk.cold[row] != 0;
+          if (p.topk.excl_off != nullptr && row_ok) {
+            int64_t lo = p.topk.excl_off[row], hi = p.topk.excl_off[row + 1];
             hend = hi;
             while (lo < hi) {
               const int64_t mid = (lo + hi) >> 1;
@@ -640,37 +627,33 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           if (topk_cnt < k) ++topk_cnt;
           if (topk_cnt == k) topk_thr = __uint_as_float(list[(k - 1) * kLs].x);
         };
-        uint32_t rbuf[2][32];
-        ptx::tmem_ld_32x32(taddr, rbuf[0]);
+        TmemChunks ch(taddr);
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
+          const uint32_t(&r)[32] = ch.wait(c, release_tmem);
           const int col0 = colh + c * 32;
-          ptx::tmem_ld_wait();
-          if (c + 1 < 4) ptx::tmem_ld_32x32(taddr + (uint32_t)((c + 1) * 32), rbuf[(c + 1) & 1]);  // prefetch
-          const uint32_t(&r)[32] = rbuf[c & 1];
-          if (c == 3) {
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) release_tmem(acc);
-          }
           if (!row_ok || col0 >= p.N) continue;
           float v[32];
           bool any = false;
 #pragma unroll
           for (int j = 0; j < 32; j += 4) {
             // scale is NaN past column N: the TMA's zero fill there never scores
-            const float4 sc = *reinterpret_cast<const float4*>(p.bias + col0 + j);
+            const float4 sc = *reinterpret_cast<const float4*>(p.topk.scale + col0 + j);
             v[j] = __uint_as_float(r[j]) * sc.x;
             v[j + 1] = __uint_as_float(r[j + 1]) * sc.y;
             v[j + 2] = __uint_as_float(r[j + 2]) * sc.z;
             v[j + 3] = __uint_as_float(r[j + 3]) * sc.w;
             if constexpr (Cfg::kBlend) {  // base is NaN past column N as well: cold rows never score the zero fill
-              const float4 b = *reinterpret_cast<const float4*>(p.topk_base + col0 + j);
-              const float a = p.topk_alpha, oma = 1.0f - p.topk_alpha;
-              v[j] = topk_cold ? b.x : v[j] * a + b.x * oma;
-              v[j + 1] = topk_cold ? b.y : v[j + 1] * a + b.y * oma;
-              v[j + 2] = topk_cold ? b.z : v[j + 2] * a + b.z * oma;
-              v[j + 3] = topk_cold ? b.w : v[j + 3] * a + b.w * oma;
+              // The fused products are spelled out, and on purpose not alike: x fuses acc * alpha, y, z and w fuse
+              // base * (1 - alpha).  That is the rounding this epilogue has always produced (the compiler used to
+              // pick it, and its pick changes with the code around it); one form for all four lanes would change
+              // scores in the last bit.
+              const float4 b = *reinterpret_cast<const float4*>(p.topk.base + col0 + j);
+              const float a = p.topk.alpha, oma = 1.0f - p.topk.alpha;
+              v[j] = topk_cold ? b.x : __fmaf_rn(v[j], a, __fmul_rn(b.x, oma));
+              v[j + 1] = topk_cold ? b.y : __fmaf_rn(b.y, oma, __fmul_rn(v[j + 1], a));
+              v[j + 2] = topk_cold ? b.z : __fmaf_rn(b.z, oma, __fmul_rn(v[j + 2], a));
+              v[j + 3] = topk_cold ? b.w : __fmaf_rn(b.w, oma, __fmul_rn(v[j + 3], a));
             }
             any |= (v[j] > topk_thr) | (v[j + 1] > topk_thr) | (v[j + 2] > topk_thr) | (v[j + 3] > topk_thr);
           }
@@ -680,53 +663,34 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           }
         }
         // segment ends (row block changes or the range ends): write the list out, padded with (NaN, -1)
-        if ((u + 1 == u_last || (u + 1) % n_units_per_row == 0) && row_ok) {
-          const int64_t c_first = ((m_u * n_units_per_row + 1) * (int64_t)n_units - 1) / total_units;
-          uint2* dst = reinterpret_cast<uint2*>(p.y) + ((row * 2 + hf) * p.ldy + ((int64_t)unit - c_first)) * k;
+        if (sched.ends_segment(u, u_last) && row_ok) {
+          const int64_t slot = (int64_t)unit - sched.first_owner(u / sched.n_per_row);
+          uint2* dst = p.topk.parts + ((row * 2 + hf) * p.topk.slots + slot) * k;
           for (int j = 0; j < k; ++j)
             dst[j] = j < topk_cnt ? list[j * kLs] : make_uint2(0x7fc00000u, 0xffffffffu);
         }
       } else if constexpr (Cfg::kStaged) {
         // ---------- element-wise epilogue, bf16 output through smem + TMA store ----------
-        uint32_t rbuf[2][32];
-        ptx::tmem_ld_32x32(taddr, rbuf[0]);
+        TmemChunks ch(taddr);
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
+          const uint32_t(&r)[32] = ch.wait(c, release_tmem);
           const int col0 = colh + c * 32;
           const bool active = col0 < p.N;  // uniform across the half
-          ptx::tmem_ld_wait();
-          if (c + 1 < 4) ptx::tmem_ld_32x32(taddr + (uint32_t)((c + 1) * 32), rbuf[(c + 1) & 1]);  // prefetch
-          const uint32_t(&r)[32] = rbuf[c & 1];
-          if (c == 3) {
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) release_tmem(acc);
-          }
           float v[32];
           if (active) activate_chunk<EPI>(r, p, row, col0, row_ok, v);
           constexpr int kChunksPerGroup = kGeglu ? 4 : 2;  // accumulator chunks that fill one 64-column group
           const int cg = c % kChunksPerGroup;
-          if (cg == 0) {
-            if (issuer) ptx::tma_store_wait_read1();
-            ptx::named_bar_sync(bar_id, 128);
-          }
-          const uint32_t stg = ptx::smem_u32(stg_base + gsel * kGroupBytes);
+          if (cg == 0) out.begin();
           if (active) {
             if (kGeglu)
-              stage_values<16>(stg, r_tile, cg * 2, v);
+              stage_values<16>(ptx::smem_u32(out.buf()), r_tile, cg * 2, v);
             else
-              stage_values<32>(stg, r_tile, cg * 4, v);
+              stage_values<32>(ptx::smem_u32(out.buf()), r_tile, cg * 4, v);
           }
           if (cg == kChunksPerGroup - 1) {
-            ptx::fence_proxy_async();
-            ptx::named_bar_sync(bar_id, 128);
             const int out_col = kGeglu ? (colh >> 1) : (colh + (c / 2) * 64);
-            const int n_out = kGeglu ? (p.N >> 1) : p.N;
-            if (issuer) {
-              if (out_col < n_out) ptx::tma_store_2d(&map_y, stg_base + gsel * kGroupBytes, out_col, m_blk * kBM);
-              ptx::tma_store_commit();  // committed even when empty: keeps the group count in step with gsel
-            }
-            gsel ^= 1;
+            out.end(&map_y, out_col < (kGeglu ? (p.N >> 1) : p.N), out_col, m_blk * kBM);
           }
         }
       } else if constexpr (Cfg::kXpose) {
@@ -738,21 +702,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         const uint32_t patch = ptx::smem_u32(xpose + e * 4096);
         const int sub_row = lane >> 3, chunk16 = lane & 7;
         const int64_t row0 = (int64_t)m_blk * kBM + quad * 32;
-        uint32_t rbuf[2][32];
-        ptx::tmem_ld_32x32(taddr, rbuf[0]);
+        TmemChunks ch(taddr);
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
+          const uint32_t(&r)[32] = ch.wait(c, release_tmem);
           const int col0 = colh + c * 32;
-          const bool active = col0 < p.N;  // warp-uniform
-          ptx::tmem_ld_wait();
-          if (c + 1 < 4) ptx::tmem_ld_32x32(taddr + (uint32_t)((c + 1) * 32), rbuf[(c + 1) & 1]);  // prefetch
-          const uint32_t(&r)[32] = rbuf[c & 1];
-          if (c == 3) {
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) release_tmem(acc);
-          }
-          if (!active) continue;
+          if (col0 >= p.N) continue;  // warp-uniform
           // residual rows of phase 2 are requested first: their latency hides behind phase 1
           uint4 rres[8];
           if (EPI == NRB_EPI_RESIDUAL) {
@@ -800,30 +755,21 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         }
       } else {
         // ---------- element-wise epilogue, fp32 output with 128-bit global stores (GEGLU + fp32 only) ----------
-#pragma unroll 1
-        for (int c = 0; c < 4; ++c) {
-          const int col0 = colh + c * 32;
-          if (col0 >= p.N) break;  // warp-uniform
-          uint32_t r[32];
-          ptx::tmem_ld_32x32(taddr + (uint32_t)(c * 32), r);
-          ptx::tmem_ld_wait();
-          if (row_ok) {
-            float v[32];
-            activate_chunk<EPI>(r, p, row, col0, row_ok, v);
-            float* y = reinterpret_cast<float*>(p.y) + row * p.ldy + (col0 >> 1);
+        TmemChunks ch(taddr);
 #pragma unroll
-            for (int j = 0; j < 16; j += 4)
-              *reinterpret_cast<float4*>(y + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-          }
+        for (int c = 0; c < 4; ++c) {
+          const uint32_t(&r)[32] = ch.wait(c, release_tmem);
+          const int col0 = colh + c * 32;
+          if (col0 >= p.N || !row_ok) continue;  // col0 >= p.N: warp-uniform
+          float v[32];
+          activate_chunk<EPI>(r, p, row, col0, row_ok, v);
+          float* y = reinterpret_cast<float*>(p.y) + row * p.ldy + (col0 >> 1);
+#pragma unroll
+          for (int j = 0; j < 16; j += 4)
+            *reinterpret_cast<float4*>(y + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
         }
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) release_tmem(acc);
       }
-      if (++acc == 2) {
-        acc = 0;
-        acc_phase ^= 1;
-      }
+      acc.advance();
     }
     if (Cfg::kStaged && issuer) ptx::tma_store_wait_all();
   }
@@ -833,10 +779,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   if (clustered) ptx::cluster_sync_all();  // no CTA may exit while a peer can still touch its smem / TMEM
   if (warp == 2) {
     ptx::tc_fence_after();
-    if (CG == 2)
-      ptx::tmem_dealloc_cg2(tmem_base, Cfg::kTmemCols);
-    else
-      ptx::tmem_dealloc(tmem_base, Cfg::kTmemCols);
+    ptx::tmem_dealloc<CG>(tmem_base, Cfg::kTmemCols);
   }
 }
 
@@ -896,9 +839,8 @@ static int launch_gemm(const CUtensorMap& ma, const CUtensorMap& mw, const CUten
     NRB_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
     if (dev >= 0 && dev < 64) attr_set[dev] = true;
   }
-  const int cs = CG == 2 ? 2 : (Cfg::kSoftmax ? p.cluster : 1);
-  const int n_split = CG == 2 ? 1 : cs;
-  const int64_t units = ((p.M + kBM * CG - 1) / (kBM * CG)) * (int64_t)(((p.N + BN - 1) / BN) / n_split);
+  const int n_split = Cfg::kSoftmax ? p.cluster : 1;  // CTAs of a softmax cluster split the N tiles of a unit
+  const int cs = CG * n_split;                         // CTAs per scheduling unit
   int max_units = sm_count_cached() / cs;
   if (cs > 1 || Cfg::kSoftmax) {  // softmax always launches as a cluster (st.async / mapa need one, even of size 1)
     cudaLaunchConfig_t cfg = {};
@@ -928,11 +870,10 @@ static int launch_gemm(const CUtensorMap& ma, const CUtensorMap& mw, const CUten
       }
       max_units = std::min(max_units, max_clusters[dev][cs]);
     }
-    const int grid = (int)std::min<int64_t>(units, max_units) * cs;
-    cfg.gridDim = dim3(grid);
+    cfg.gridDim = dim3((int)TileSchedule(p.M, p.N, BN, CG, n_split, max_units).n_ctas * cs);
     NRB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kern, ma, mw, my, p));
   } else {
-    const int grid = (int)std::min<int64_t>(units, max_units);
+    const int grid = (int)TileSchedule(p.M, p.N, BN, CG, 1, max_units).n_ctas;
     kern<<<grid, kGemmThreads, Cfg::kSmemBytes, st>>>(ma, mw, my, p);
   }
   note_launch();
@@ -989,12 +930,8 @@ int gemm_bf16_tc(int epi, int out_dtype, const void* a, int64_t lda, const void*
   }
   const bool small_n = N <= 128 && !softmax;
   // CTA pairs (tcgen05 cta_group::2): each SM stages only half of the W tile -> 1/3 less shared-memory
-  // operand traffic per MMA.  NRB200_GEMM_2CTA=0 selects the single-CTA kernel.
-  static const bool pair_enabled = [] {
-    const char* e = getenv("NRB200_GEMM_2CTA");
-    return e == nullptr || e[0] != '0';
-  }();
-  const bool pair = pair_enabled && !small_n && !softmax && M > kBM;
+  // operand traffic per MMA
+  const bool pair = !small_n && !softmax && M > kBM;
   CUtensorMap ma, mw, my;
   int rc = make_tmap_bf16(&ma, a, M, K, lda, kBM);
   if (rc != NRB_OK) return rc;
@@ -1036,25 +973,16 @@ int gemm_bf16_tc(int epi, int out_dtype, const void* a, int64_t lda, const void*
                                : dispatch_epi<256, false>(epi, ma, mw, my, p, st);
 }
 
-// Schedule of the top-k GEMM, computed the way launch_gemm sizes its grid: `units` scheduling units (one 128-row block,
-// or 256 rows on a CTA pair, times one 256-column tile) split into contiguous ranges over `n_units` CTAs (pairs);
-// `slots` = the most CTAs whose range touches one row block, i.e. the partial lists each (row, half) may get.
+// The schedule launch_gemm gives the top-k GEMM
 TopkPlan topk_plan(int64_t M, int64_t N) {
-  TopkPlan t;
-  t.cg = M > kBM ? 2 : 1;
-  t.rows_per_block = kBM * t.cg;
-  t.m_tiles = (M + t.rows_per_block - 1) / t.rows_per_block;
-  t.n_per_row = (N + 255) / 256;
-  t.units = t.m_tiles * t.n_per_row;
-  t.n_units = std::min<int64_t>(t.units, sm_count_cached() / t.cg);
-  t.slots = 1;
-  for (int64_t m = 0; m < t.m_tiles; ++m)
-    t.slots = std::max(t.slots, topk_owner(t, (m + 1) * t.n_per_row - 1) - topk_owner(t, m * t.n_per_row) + 1);
+  const int cg = M > kBM ? 2 : 1;
+  TopkPlan t{TileSchedule(M, (int)N, 256, cg, 1, sm_count_cached() / cg), 1};
+  for (int64_t m = 0; m < t.m_blocks; ++m) t.slots = std::max(t.slots, t.last_owner(m) - t.first_owner(m) + 1);
   return t;
 }
 
 // Partial top-k lists of (a[M,K] . w[N,K]^T) * scale[N] per row, blended with base[N] when base != NULL: see
-// GemmParams for the NRB_EPI_TOPK / NRB_EPI_TOPK_BLEND fields.
+// GemmParams::TopkArgs.
 int gemm_topk_tc(const void* a, int64_t lda, const void* w, int64_t ldw, const float* scale, const int64_t* excl_off,
                  const int32_t* excl_sorted, int64_t M, int N, int K, int k, const TopkPlan& plan, void* parts,
                  const float* base, const uint8_t* cold, float alpha, cudaStream_t st) {
@@ -1065,24 +993,12 @@ int gemm_topk_tc(const void* a, int64_t lda, const void* w, int64_t ldw, const f
   if (rc != NRB_OK) return rc;
   rc = make_tmap_bf16(&mw, w, N, K, ldw, plan.cg == 2 ? 128 : 256);
   if (rc != NRB_OK) return rc;
-  GemmParams p = {};
+  GemmParams p = {};  // no all-gather rides along: it rides on the dense row kernels only
   p.M = M;
-  p.m_dev = nullptr;
   p.N = N;
   p.K = K;
-  p.bias = scale;
-  p.res = excl_off;
-  p.res_dtype = NRB_F32;
-  p.res_map = excl_sorted;
-  p.y = parts;
-  p.ldy = plan.slots;
-  p.group = k;
-  p.cluster = 1;
-  p.push.n_seg = 0;  // the all-gather rides on the dense row kernels only
+  p.topk = {scale, excl_off, excl_sorted, static_cast<uint2*>(parts), plan.slots, k, base, cold, alpha};
   if (base != nullptr) {
-    p.topk_base = base;
-    p.topk_cold = cold;
-    p.topk_alpha = alpha;
     if (plan.cg == 2) return launch_gemm<256, NRB_EPI_TOPK_BLEND, false, 2>(ma, mw, ma, p, st);
     return launch_gemm<256, NRB_EPI_TOPK_BLEND, false, 1>(ma, mw, ma, p, st);
   }

@@ -1,5 +1,6 @@
 // Thin inline-PTX wrappers for the Blackwell (sm_100a) async machinery used by the dense
-// kernels: mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (MMA / TMEM alloc / ld / commit).
+// kernels: mbarrier, TMA (cp.async.bulk.tensor), tcgen05 (MMA / TMEM alloc / ld / commit), clusters.
+// The wrappers templated on CG issue the cta_group::CG form: CG = 2 is a CTA pair whose MMA spans both SMs.
 #pragma once
 
 #include <cuda.h>
@@ -12,6 +13,8 @@ namespace ptx {
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
+// shared::cluster address of the same smem offset in the even (leader) CTA of a CTA pair
+__device__ __forceinline__ uint32_t leader_addr(uint32_t smem_addr) { return smem_addr & 0xFEFFFFFFu; }
 
 // ---- mbarrier -------------------------------------------------------------------------
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
@@ -47,27 +50,45 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   while (!mbar_try_wait(bar, parity)) {
   }
 }
+// remote arrive WITHOUT a memory release: enough when the ordering that matters is carried by tcgen05 fences
+__device__ __forceinline__ void mbar_arrive_cluster_relaxed(uint32_t cluster_bar_addr) {
+  asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar_addr) : "memory");
+}
 
 // ---- TMA ------------------------------------------------------------------------------
 __device__ __forceinline__ void prefetch_tensormap(const CUtensorMap* m) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
 }
-// 2-D tiled load global -> shared, completion counted in bytes on `bar`.
-__device__ __forceinline__ void tma_load_2d(void* dst_smem, const CUtensorMap* map, uint64_t* bar, int c0,
-                                            int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst_smem)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-      : "memory");
+// 2-D tiled load global -> this CTA's shared memory, completion counted in bytes on `bar` (CG = 2: on the barrier at
+// the same offset in the leader CTA)
+template <int CG>
+__device__ __forceinline__ void tma_load_2d(void* dst_smem, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
+  if constexpr (CG == 1)
+    asm volatile(
+        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+        ::"r"(smem_u32(dst_smem)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
+        : "memory");
+  else
+    asm volatile(
+        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+        ::"r"(smem_u32(dst_smem)), "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_addr(smem_u32(bar))), "r"(c0),
+        "r"(c1)
+        : "memory");
 }
-__device__ __forceinline__ void tma_load_2d_hint(void* dst_smem, const CUtensorMap* map, uint64_t* bar, int c0,
-                                                 int c1, uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint "
-      "[%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(dst_smem)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1),
-      "l"(policy)
-      : "memory");
+// TMA store shared -> global (bulk async group)
+__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* src_smem, int c0, int c1) {
+  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
+                   reinterpret_cast<uint64_t>(map)),
+               "r"(smem_u32(src_smem)), "r"(c0), "r"(c1)
+               : "memory");
+}
+__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// at most one committed group may still be reading its smem (double-buffered staging)
+__device__ __forceinline__ void tma_store_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
+__device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+
+__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
 // ---- tcgen05 ----------------------------------------------------------------------------
@@ -75,34 +96,70 @@ __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence:
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
 // whole warp; writes the TMEM base address to *dst_smem
+template <int CG>
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)),
-               "r"(ncols)
-               : "memory");
+  if constexpr (CG == 1)
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)),
+                 "r"(ncols)
+                 : "memory");
+  else
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)),
+                 "r"(ncols)
+                 : "memory");
 }
+template <int CG>
 __device__ __forceinline__ void tmem_relinquish() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  if constexpr (CG == 1)
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  else
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
 }
+template <int CG>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+  if constexpr (CG == 1)
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+  else
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
 
 // D[tmem] (+)= A[smem] * B[smem]^T, bf16 inputs, fp32 accumulate; single issuing thread.
+// CG = 2: D in the TMEM of both CTAs, A from each CTA's smem, the N rows of B split over both CTAs' smem; issued by
+// the leader only.
+template <int CG>
 __device__ __forceinline__ void mma_bf16_ss(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
                                             uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
+  if constexpr (CG == 1)
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
+        "}"
+        ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+        : "memory");
+  else
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
+        "}"
+        ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+        : "memory");
 }
-// arrive on `bar` once all previously issued MMAs of this thread have completed
+// arrive on `bar` (CG = 2: on the barrier at this smem offset in BOTH CTAs of the pair) once all previously issued
+// MMAs of this thread have completed
+template <int CG>
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
+  if constexpr (CG == 1)
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
+                 : "memory");
+  else
+    asm volatile(
+        "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+            smem_u32(bar)),
+        "h"((uint16_t)3)
+        : "memory");
 }
 
 // TMEM -> registers: 32 lanes (this warp's quadrant) x 32 consecutive fp32 columns.
@@ -154,43 +211,6 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(int m, int n) {
          | ((uint32_t)(m >> 4) << 24);  // M >> 4
 }
 
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred = 0;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred P;\n\t"
-      "elect.sync _|P, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, P;\n\t"
-      "}"
-      : "=r"(pred));
-  return pred != 0;
-}
-
-}  // namespace ptx
-}  // namespace nrb
-
-// ---- additions for the staged-store / cluster epilogues ------------------------------------
-namespace nrb {
-namespace ptx {
-
-// TMA store shared -> global (bulk async group)
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* src_smem, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(map)),
-               "r"(smem_u32(src_smem)), "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// smem of all committed groups has been read (safe to overwrite the staging buffer)
-__device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-// at most one committed group may still be reading its smem (double-buffered staging)
-__device__ __forceinline__ void tma_store_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
-__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
-
 // ---- thread-block cluster / distributed shared memory --------------------------------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
@@ -216,9 +236,6 @@ __device__ __forceinline__ uint32_t map_to_cta(uint32_t local_smem_addr, uint32_
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_smem_addr), "r"(rank));
   return r;
 }
-__device__ __forceinline__ void st_cluster_f32(uint32_t cluster_addr, float v) {
-  asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(cluster_addr), "f"(v) : "memory");
-}
 // asynchronous DSMEM store of two floats; completion is counted (8 bytes) on the DESTINATION CTA's mbarrier,
 // so the producer needs no release fence and the consumer's mbarrier wait makes the data visible
 __device__ __forceinline__ void st_async_v2_f32(uint32_t cluster_addr, float a, float b, uint32_t cluster_bar_addr) {
@@ -226,77 +243,6 @@ __device__ __forceinline__ void st_async_v2_f32(uint32_t cluster_addr, float a, 
                    cluster_addr),
                "f"(a), "f"(b), "r"(cluster_bar_addr)
                : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_bar_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar_addr) : "memory");
-}
-// remote arrive WITHOUT a memory release: enough when the ordering that matters is carried by tcgen05 fences
-__device__ __forceinline__ void mbar_arrive_cluster_relaxed(uint32_t cluster_bar_addr) {
-  asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-  }
-}
-
-}  // namespace ptx
-}  // namespace nrb
-
-// ---- cta_group::2 (CTA pair) variants ------------------------------------------------------------------
-namespace nrb {
-namespace ptx {
-
-// shared::cluster address of the same smem offset in the even (leader) CTA of a CTA pair
-__device__ __forceinline__ uint32_t leader_addr(uint32_t smem_addr) { return smem_addr & 0xFEFFFFFFu; }
-
-// 2-D tiled load into THIS CTA's smem; the transaction bytes are counted on the leader CTA's mbarrier
-__device__ __forceinline__ void tma_load_2d_cg2(void* dst_smem, const CUtensorMap* map, uint32_t leader_bar, int c0,
-                                                int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst_smem)), "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_cg2(uint32_t* dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)),
-               "r"(ncols)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_cg2() {
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_cg2(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// D[tmem of both CTAs] (+)= A[each CTA's smem] * B[N split over both CTAs' smem]^T; issued by the leader only
-__device__ __forceinline__ void mma_bf16_ss_cg2(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                                uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive on the barrier at this smem offset in BOTH CTAs of the pair once the MMAs issued so far have completed
-__device__ __forceinline__ void mma_commit_cg2(uint64_t* bar) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"((uint16_t)3)
-      : "memory");
 }
 
 }  // namespace ptx

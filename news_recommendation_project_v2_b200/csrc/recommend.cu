@@ -204,9 +204,9 @@ merge_kernel(const uint2* parts, TopkPlan plan, int64_t n_users, int k, const in
   if (u >= n_users) return;
   const int64_t S = plan.slots;
   int32_t* heads = heads_all + (int64_t)w * 2 * S;
-  const int64_t m_u = u / plan.rows_per_block;
-  const int64_t c_first = topk_owner(plan, m_u * plan.n_per_row);
-  const int n_used = (int)(topk_owner(plan, (m_u + 1) * plan.n_per_row - 1) - c_first + 1);
+  const int64_t m_u = u / (128 * plan.cg);
+  const int64_t c_first = plan.first_owner(m_u);
+  const int n_used = (int)(plan.last_owner(m_u) - c_first + 1);
   const int n_lists = 2 * n_used;
   auto list_base = [&](int i) {  // list i = (half i / n_used, slot i % n_used)
     return parts + ((u * 2 + i / n_used) * S + (i % n_used)) * k;
@@ -274,7 +274,7 @@ static RecLayout rec_layout(void* base, int precision, int dim, int64_t n_users,
   L.cold = (uint8_t*)ws.take((size_t)n_users);
   L.excl_sorted = (int32_t*)ws.take((size_t)std::max<int64_t>(n_excl, 1) * 4);
   L.excl_tmp = (int32_t*)ws.take((size_t)std::max<int64_t>(n_excl, 1) * 4);
-  L.parts = (uint2*)ws.take((size_t)plan.m_tiles * plan.rows_per_block * 2 * plan.slots * k * 8);
+  L.parts = (uint2*)ws.take((size_t)plan.m_blocks * 128 * plan.cg * 2 * plan.slots * k * 8);
   L.bytes = ws.used + 256;
   return L;
 }

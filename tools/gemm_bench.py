@@ -1,6 +1,6 @@
 """Micro-benchmark of the tcgen05 dense row kernel (nrb_linear) on the shapes the hot path uses.
 
-    python tools/gemm_bench.py [tag]        # NRB200_GEMM_2CTA=0 selects the single-CTA (cta_group::1) kernel
+    python tools/gemm_bench.py [tag]
 """
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
